@@ -50,6 +50,7 @@ OPS_PER_DESC_PAIR = 256               # 128 MAC
 SWEEP_CAMS = (50, 100, 200, 500, 2000)
 CPU_MATCH_IMAGES = 26                 # 325 pairs of 5000 x 5000: ~3 s of the reference on a 128-thread host
 GEOM_PAIRS, GEOM_MATCHES = 2000, 800  # geometric-filter leg: pairs x putative matches per pair
+DUMP_BYTES = 60 << 20                 # --dump-outputs budget (array data), under 64 MB with the .npy headers
 
 
 def peaks():
@@ -109,6 +110,19 @@ def pair_shard(pi, pj, rank, world):
     return np.ascontiguousarray(pi[sl]), np.ascontiguousarray(pj[sl])
 
 
+def dump_outputs(path, arrays):
+    """Write each array as <path>/<name>.npy.  Smallest first; an array larger than what is left of DUMP_BYTES is
+    replaced by a fixed, seeded sample of its rows (the same rows for the same shape), so two builds compare row for row."""
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_BYTES
+    for name, a in sorted(arrays.items(), key=lambda kv: kv[1].nbytes):
+        if a.nbytes > left:
+            keep = left // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
+
+
 # ===================================================================================== ours (GPU)
 def run_ours(args):
     import torch
@@ -141,6 +155,7 @@ def run_ours(args):
     pk = peaks()
     K, W = args.steps, args.warmup
     launches = 0
+    outputs = {}                                      # what the last timed step of each leg returned (--dump-outputs)
     # ------------------------------------------------------------------ BA (replica per rank, same scene)
     scene = synth.ba_scene(*BA_CFG, seed=BA_SEED)
     n_obs = len(scene["obs_view"])
@@ -159,6 +174,9 @@ def run_ours(args):
     ba_time = allmax(max(dev_ms / 1e3, 0.0))
     ba_wall = allmax(wall)
     ba_iters_all = allsum(iters)
+    if args.dump_outputs:
+        poses, intr, pts = ctx.download()
+        outputs.update(ba_poses=poses, ba_intrinsics=intr, ba_points=pts, ba_cost=np.array([last["initial_cost"], last["final_cost"]]))
     ctx.close()
     # e2e: host buffers in, host buffers out, everything inside the timed region
     barrier()
@@ -222,7 +240,7 @@ def run_ours(args):
         launches += 1
 
     # ------------------------------------------------------------------ MATCH (pairs sharded over ranks)
-    def match_leg(n_img, steps, warm, e2e_steps, with_cascade):
+    def match_leg(n_img, steps, warm, e2e_steps, with_cascade, keep_outputs=False):
         nonlocal launches
         lo, hi, per = image_shard(n_img, rank, world)
         mine = synth.descriptor_collection(n_img, MATCH_DESC, seed=MATCH_SEED, lo=lo, hi=hi)
@@ -264,6 +282,8 @@ def run_ours(args):
         tc_ms, tc_n = mctx.kernel_time(reset=True)
         off, ij = mctx.fetch()
         n_matches = len(ij)
+        if keep_outputs:                              # indices below 2^24 (float32) and offsets below 2^53 (float64) stay exact
+            outputs.update(match_offsets=off.astype(np.float64), match_ij=ij.astype(np.float32))
         # e2e: descriptors start in pinned host memory (this rank's 1/N); copy + all-gather + arena + prepare + run + fetch timed
         ag_ms.clear()
         barrier(); t0 = time.perf_counter()
@@ -318,7 +338,7 @@ def run_ours(args):
         return res
 
     n_img = MATCH_IMAGES if args.match_images is None else args.match_images
-    match = match_leg(n_img, K, W, max(1, min(K, 3)), True)
+    match = match_leg(n_img, K, W, max(1, min(K, 3)), True, keep_outputs=bool(args.dump_outputs))
     clk.__exit__()
     m2 = None
     if args.m2 or (world == 8 and not args.no_m2):
@@ -345,6 +365,8 @@ def run_ours(args):
         if not args.no_cpu and world == 1:
             cb, mb, _ = cpu_baselines(scene, full=False)
             line["cpu_baseline"], line["match"]["cpu_baseline"] = cb, mb
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -462,7 +484,14 @@ def main():
     ap.add_argument("--no-m2", action="store_true")
     ap.add_argument("--match-images", type=int, default=None)
     ap.add_argument("--quick", action="store_true", help="--impl reference only: one thread count, 15-pair MATCH sample, no sweep (the CPU test-suite uses it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last BA solve and the last MATCH pass returned as DIR/<name>.npy "
+                         "(float64 / float32, at most 64 MB; with --gpus N > 1, rank 0's pair shard of MATCH)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours" and not args.no_cpu:
         args.warmup = 3
     if args.impl == "reference":

@@ -2,6 +2,7 @@
 oracle/Makefile from /root/reference sources in place) on seeded inputs from openmvg_b200.synth.
 Run in the build container:  python tests/golden/make_golden.py
 The inputs are regenerated from their seeds at test time; only the reference's outputs are stored."""
+import hashlib
 import json
 import os
 import sys
@@ -197,6 +198,74 @@ def main_geom():
     json.dump(out, open(path, "w"), indent=1)
 
 
+# What the oracle tests (tests/test_oracle_{ba,match,geom}.py) compare against when they check the oracle case by
+# case: the reference's own results on the same seeded inputs, so those comparisons run without the reference.
+ORACLE_BA_KW = [dict(), dict(intrinsics_opt=1), dict(extrinsics_opt=4), dict(structure_opt=0)]
+ORACLE_BA_EXT_KW = [dict(intrinsics_opt=1), dict(extrinsics_opt=4), dict(structure_opt=0), dict(use_loss=0), dict(model=3)]
+
+
+def kw_key(kw):
+    return "_".join(f"{a}{b}" for a, b in kw.items()) or "default"
+
+
+def main_oracle_cases():
+    out = {}
+
+    def put(prefix, **arrays):
+        for k, v in arrays.items():
+            out[f"{prefix}.{k}"] = np.asarray(v)
+
+    def registered(prefix, s, **ref_kw):
+        r = ck.ref_ba_adjust_ex(s, **ref_kw)
+        t, fit, cen = ck.ref_ba_register_priors(s)
+        put(prefix, ok=r["ok"], final_cost=r["final_cost"], iterations=r["iterations"], points=r["points"], prior_fit=r["prior_fit"],
+            reg_poses=t["poses"], reg_points=t["points"], reg_prior_center=t["prior_center"], reg_fit=fit, reg_centroid=cen)
+
+    for kw in ORACLE_BA_KW:
+        r = ck.ref_ba_adjust(synth.ba_scene(12, 400, 5, seed=13, outlier_frac=0.01), threads=2, **kw)
+        put("ba." + kw_key(kw), ok=r["ok"], final_cost=r["final_cost"], iterations=r["iterations"], poses=r["poses"], points=r["points"])
+    registered("ba_ext", synth.add_priors(synth.add_gcp(synth.ba_scene(12, 300, 5, seed=3), 6, weight=15.0), sigma=0.02))
+    for kw in ORACLE_BA_EXT_KW:
+        kw = dict(kw); model = kw.pop("model", 1)
+        s = synth.add_priors(synth.add_gcp(synth.ba_scene(14, 400, 5, seed=6, model=model), 5, weight=12.0), sigma=0.015)
+        registered("ba_ext." + kw_key(kw or dict(model=model)), s, **kw)
+
+    descs = synth.descriptors(4, [257, 300, 64, 129], seed=77)
+    pi, pj = np.meshgrid(np.arange(4), np.arange(4), indexing="ij")
+    keep = pi != pj
+    pi = pi[keep].astype(np.uint32); pj = pj[keep].astype(np.uint32)
+    order = np.lexsort((pj, pi)); pi, pj = pi[order], pj[order]
+    for ratio in (0.8, 0.95, 0.5):
+        roff, rij = ck.ref_match_collection(descs, pi, pj, ratio)
+        put(f"match.{ratio}", offsets=roff, ij=rij)
+    put("match", pair01=ck.ref_match_pair(descs[0], descs[1]))
+
+    descs = synth.descriptors(3, [1200, 1000, 700], seed=21)
+    P, S = ck.ref_cascade_projections()
+    put("cascade", projections_sha256=np.frombuffer(hashlib.sha256(P.tobytes() + S.tobytes()).digest(), np.uint8),
+        zero_mean=ck.ref_cascade_zero_mean(descs, [0, 1, 2]))
+    for k, d in enumerate(descs):
+        codes, bids = ck.ref_cascade_hash(d, out["cascade.zero_mean"])
+        put(f"cascade.{k}", codes=codes, bids=bids)
+    roff, rij = ck.ref_cascade_collection(descs, *synth.exhaustive_pairs(3), 0.8)
+    put("cascade", offsets=roff, ij=rij)
+
+    for seed in range(20, 32):
+        rng = np.random.default_rng(seed)
+        n = int(rng.integers(9, 900)); of = float(rng.uniform(0.0, 0.7)); it = int(rng.choice([64, 256, 2048]))
+        xI, xJ, _ = synth.two_view_matches(n, of, seed=seed, wh=(1600, 1200))
+        r = ck.ref_acransac_fundamental(xI, xJ, (1600, 1200, 1600, 1200), 4.0, it)
+        put(f"geom_F.{seed}", inliers=r["inliers"], error_max=r["error_max"], min_nfa=r["min_nfa"])
+    for seed in range(40, 48):
+        rng = np.random.default_rng(seed)
+        n = int(rng.integers(5, 900)); of = float(rng.uniform(0.0, 0.7)); it = int(rng.choice([64, 2048]))
+        xI, xJ, _ = synth.two_view_matches(n, of, seed=seed, wh=(1600, 1200), planar=True)
+        r = ck.ref_acransac_homography(xI, xJ, (1600, 1200, 1600, 1200), 4.0, it)
+        put(f"geom_H.{seed}", inliers=r["inliers"], min_nfa=r["min_nfa"])
+    np.savez_compressed(os.path.join(HERE, "reference_oracle_cases.npz"), **out)
+    print("oracle cases", len(out), "arrays")
+
+
 def main():
     out = {"match": [], "ba": []}
     arrays = {}
@@ -232,6 +301,8 @@ if __name__ == "__main__":
         main_more()
     elif len(sys.argv) > 1 and sys.argv[1] == "geom":
         main_geom()
+    elif len(sys.argv) > 1 and sys.argv[1] == "oracle_cases":
+        main_oracle_cases()
     else:
         main()
         main_ext()

@@ -106,6 +106,22 @@ def test_pair_sharding_world2_gloo(tmp_path):
         assert p.returncode == 0, o
 
 
+def test_bench_dump_outputs_budget_and_sample(tmp_path):
+    """bench.py --dump-outputs: one .npy per array, at most 64 MB in all; an array over the budget becomes a seeded
+    sample of its rows, the same rows on every run."""
+    import bench
+    small = np.linspace(0.0, 1.0, 7)
+    big = np.arange(3 * bench.DUMP_BYTES // 8, dtype=np.float32).reshape(-1, 2)        # 1.5 x the budget
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"small": small, "big": big})
+    assert sorted(os.listdir(tmp_path / "a")) == ["big.npy", "small.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64_000_000
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), small)
+    s = np.load(tmp_path / "a" / "big.npy")
+    assert s.dtype == np.float32 and 0 < len(s) < len(big) and np.all(np.diff(s[:, 0]) > 0) and np.array_equal(s, big[(s[:, 0] // 2).astype(np.int64)])
+    assert np.array_equal(s, np.load(tmp_path / "b" / "big.npy"))
+
+
 # ---- file formats (SURVEY §8f N3): host-side, no GPU needed
 def _sample_csr():
     pI = np.array([7, 2, 2, 9, 4], np.uint32); pJ = np.array([9, 5, 3, 11, 6], np.uint32)      # unsorted, one empty pair

@@ -1,16 +1,21 @@
 """CPU: the BA oracle against the committed golden outputs of the reference's own
-Bundle_Adjustment_Ceres::Adjust (tests/golden/reference_outputs.json) and, when oracle/_ref is
-present, the compiled reference itself."""
+Bundle_Adjustment_Ceres::Adjust (tests/golden/reference_outputs.json, reference_oracle_cases.npz)."""
 import json
 import os
+import sys
 
 import numpy as np
 import pytest
 
 import checkers as ck
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+from make_golden import ORACLE_BA_EXT_KW, ORACLE_BA_KW, kw_key
 from openmvg_b200 import synth
 
-GOLD = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "reference_outputs.json")))
+G = os.path.join(os.path.dirname(__file__), "golden")
+GOLD = json.load(open(os.path.join(G, "reference_outputs.json")))
+REF = np.load(os.path.join(G, "reference_oracle_cases.npz"))
 SMALL = [c for c in GOLD["ba"] if c["scene"]["n_cams"] <= 100]
 
 
@@ -52,11 +57,24 @@ def test_jacobian_against_finite_differences():
             assert np.abs(fd - J[:, :, k]).max() <= 2e-4 * max(1.0, np.abs(J[:, :, k]).max()), (name, k)
 
 
-@pytest.mark.skipif(not ck.have_ref_ba(), reason="oracle/_ref not built (no /root/reference here)")
-@pytest.mark.parametrize("kw", [dict(), dict(intrinsics_opt=1), dict(extrinsics_opt=4), dict(structure_opt=0)])
+def reference_case(prefix):
+    """The reference's results for one case of tests/golden/reference_oracle_cases.npz (make_golden.py oracle_cases)."""
+    return {k[len(prefix) + 1:]: REF[k] for k in REF.files if k.startswith(prefix + ".") and "." not in k[len(prefix) + 1:]}
+
+
+def registered_scene(s, r):
+    """The scene after the reference's pre-solve registration of the priors (ck.ref_ba_register_priors)."""
+    t = dict(s)
+    if r["reg_fit"] >= 0:
+        t.update(poses=r["reg_poses"].copy(), points=r["reg_points"].copy(), prior_center=r["reg_prior_center"].copy(),
+                 prior_huber_a=float(r["reg_fit"]) ** 2)
+    return t
+
+
+@pytest.mark.parametrize("kw", ORACLE_BA_KW)
 def test_against_compiled_reference(kw):
     s = synth.ba_scene(12, 400, 5, seed=13, outlier_frac=0.01)
-    r = ck.ref_ba_adjust(s, threads=2, **kw)
+    r = reference_case("ba." + kw_key(kw))
     o = ck.oracle_ba_solve(s, **kw)
     assert r["ok"] and o["usable"]
     assert abs(o["final_cost"] - r["final_cost"]) <= 1e-9 * r["final_cost"]
@@ -84,11 +102,10 @@ def test_golden_gcp_and_priors(case):
     assert abs(ck.oracle_ba_cost(ret, use_loss=case["opts"].get("use_loss", 1)) - o["final_cost"]) <= 1e-12 * o["final_cost"]
 
 
-@pytest.mark.skipif(not ck.have_ref_ba(), reason="oracle/_ref not built")
 def test_gcp_and_priors_against_compiled_reference():
     s = synth.add_priors(synth.add_gcp(synth.ba_scene(12, 300, 5, seed=3), 6, weight=15.0), sigma=0.02)   # GCPs live in the priors' frame
-    r = ck.ref_ba_adjust_ex(s)
-    t, fit, cen = ck.ref_ba_register_priors(s)
+    r = reference_case("ba_ext")
+    t, fit, cen = registered_scene(s, r), r["reg_fit"], r["reg_centroid"]
     assert fit == r["prior_fit"] and fit > 0
     o = ck.oracle_ba_solve(t)
     assert abs(o["final_cost"] - r["final_cost"]) <= 1e-9 * r["final_cost"]
@@ -108,16 +125,13 @@ def test_zero_weight_removes_observation_exactly():
     assert abs(a["final_cost"] - b["final_cost"]) <= 1e-9 * b["final_cost"] and a["iterations"] == b["iterations"]   # (OpenMP atomics reorder sums)
 
 
-@pytest.mark.skipif(not ck.have_ref_ba(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("kw", [dict(intrinsics_opt=1), dict(extrinsics_opt=4), dict(structure_opt=0), dict(use_loss=0), dict(model=3)],
-                         ids=lambda k: "_".join(f"{a}{b}" for a, b in k.items()))
+@pytest.mark.parametrize("kw", ORACLE_BA_EXT_KW, ids=kw_key)
 def test_gcp_priors_option_mixes_against_compiled_reference(kw):
     """Control points + motion priors under the option mixes of Optimize_Options and another camera model."""
+    r = reference_case("ba_ext." + kw_key(kw))
     kw = dict(kw); model = kw.pop("model", 1)
     s = synth.add_priors(synth.add_gcp(synth.ba_scene(14, 400, 5, seed=6, model=model), 5, weight=12.0), sigma=0.015)
-    ref_kw = {k: v for k, v in kw.items() if k in ("intrinsics_opt", "extrinsics_opt", "structure_opt", "use_loss")}
-    r = ck.ref_ba_adjust_ex(s, **ref_kw)
-    t, fit, cen = ck.ref_ba_register_priors(s)
+    t = registered_scene(s, r)
     o = ck.oracle_ba_solve(t, **kw)
     assert r["ok"] and o["usable"]
     assert abs(o["final_cost"] - r["final_cost"]) <= 1e-8 * r["final_cost"], (o["final_cost"], r["final_cost"])

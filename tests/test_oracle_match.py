@@ -1,5 +1,6 @@
-"""CPU: the MATCH oracle against the reference's known answers, the committed golden vectors
-(generated from the compiled reference) and — when oracle/_ref is present — the reference itself."""
+"""CPU: the MATCH oracle against the reference's known answers and the committed golden vectors
+(generated from the compiled reference)."""
+import hashlib
 import json
 import os
 
@@ -12,6 +13,7 @@ from openmvg_b200 import synth
 G = os.path.join(os.path.dirname(__file__), "golden")
 GOLD = json.load(open(os.path.join(G, "reference_outputs.json")))
 GOLD_IJ = np.load(os.path.join(G, "reference_matches.npz"))
+REF = np.load(os.path.join(G, "reference_oracle_cases.npz"))
 
 
 def test_l2_known_answer():
@@ -72,8 +74,8 @@ def test_golden_collections(case):
         assert np.array_equal(ij, GOLD_IJ[key])
 
 
-@pytest.mark.skipif(not ck.have_ref_match(), reason="oracle/_ref not built (no /root/reference here)")
 def test_against_compiled_reference():
+    """Against the reference's Matcher_Regions on the same collection (tests/golden/reference_oracle_cases.npz)."""
     descs = synth.descriptors(4, [257, 300, 64, 129], seed=77)
     pi, pj = np.meshgrid(np.arange(4), np.arange(4), indexing="ij")
     keep = pi != pj
@@ -81,10 +83,10 @@ def test_against_compiled_reference():
     # Pair_Set is an ordered set: present pairs in sorted order to both
     order = np.lexsort((pj, pi)); pi, pj = pi[order], pj[order]
     for ratio in (0.8, 0.95, 0.5):
-        roff, rij = ck.ref_match_collection(descs, pi, pj, ratio)
+        roff, rij = REF[f"match.{ratio}.offsets"], REF[f"match.{ratio}.ij"]
         ooff, oij = ck.oracle_match_collection(descs, pi, pj, ratio)
         assert np.array_equal(roff, ooff) and np.array_equal(rij, oij)
-    a = ck.ref_match_pair(descs[0], descs[1]); b = ck.oracle_match_pair(descs[0], descs[1])
+    a = REF["match.pair01"]; b = ck.oracle_match_pair(descs[0], descs[1])
     assert np.array_equal(a, b)
 
 
@@ -114,24 +116,24 @@ def test_cascade_golden(case):
     assert tot > 0 or case["n_matches"] == 0
 
 
-@pytest.mark.skipif(not ck.have_ref_match(), reason="oracle/_ref not built")
 def test_cascade_stages_against_compiled_reference():
+    """Stage by stage against the reference's CascadeHasher (tests/golden/reference_oracle_cases.npz)."""
     descs = synth.descriptors(3, [1200, 1000, 700], seed=21)
-    P, S = ck.ref_cascade_projections()
-    Pg, Sg = ck.cascade_projections()
-    assert np.array_equal(P, Pg) and np.array_equal(S, Sg)            # the committed fixture is the reference's draw
+    P, S = ck.cascade_projections()
+    digest = np.frombuffer(hashlib.sha256(P.tobytes() + S.tobytes()).digest(), np.uint8)
+    assert np.array_equal(digest, REF["cascade.projections_sha256"])   # the committed fixture is the reference's draw
     used = [0, 1, 2]
-    zo = ck.oracle_cascade_zero_mean(descs, used); zr = ck.ref_cascade_zero_mean(descs, used)
+    zo = ck.oracle_cascade_zero_mean(descs, used); zr = REF["cascade.zero_mean"]
     assert np.array_equal(zo, zr)
     bits = diff = 0
-    for d in descs:
-        co, bo = ck.oracle_cascade_hash(d, zr, P, S); cr, br = ck.ref_cascade_hash(d, zr)
+    for k, d in enumerate(descs):
+        co, bo = ck.oracle_cascade_hash(d, zr, P, S); cr, br = REF[f"cascade.{k}.codes"], REF[f"cascade.{k}.bids"]
         diff += sum(bin(int(x)).count("1") for x in (co ^ cr).ravel()) + sum(bin(int(x)).count("1") for x in (bo ^ br).ravel())
         bits += co.size * 32 + bo.size * 10
     assert diff <= 1e-5 * bits, (diff, bits)
     pi, pj = synth.exhaustive_pairs(3)
     off, ij, _, _ = ck.oracle_cascade_collection(descs, pi, pj, 0.8, P, S)
-    roff, rij = ck.ref_cascade_collection(descs, pi, pj, 0.8)
+    roff, rij = REF["cascade.offsets"], REF["cascade.ij"]
     same = tot = 0
     for p in range(len(pi)):
         a = set(map(tuple, _sorted_rows(off, ij, p))); b = set(map(tuple, rij[int(roff[p]):int(roff[p + 1])]))
