@@ -96,8 +96,6 @@ int omvg_match_kernel_time(omvg_match_ctx *ctx, double *ms, uint64_t *launches, 
  * the per-accumulator key arithmetic (any uint8 descriptors; also forced by OMVG_MATCH_TC4=1), 0 = not prepared.
  * Both give bit-identical matches. */
 int omvg_match_kernel_variant(const omvg_match_ctx *ctx);
-/* CTA pairs (2-CTA clusters) that can be resident at once on this device for the cta_group::2 kernel (diagnostic). */
-int omvg_match_max_clusters(const omvg_match_ctx *ctx);
 
 /* ---- cascade hashing: openMVG's default matcher for scalar descriptors ("FASTCASCADEHASHINGL2",
  * matching/cascade_hasher.hpp, matching_image_collection/Cascade_Hashing_Matcher_Regions.cpp:38-226).

@@ -28,8 +28,6 @@ def lib() -> ctypes.CDLL:
         L.omvg_match_launch_count.argtypes = [ctypes.c_void_p]
         L.omvg_match_kernel_variant.restype = ctypes.c_int
         L.omvg_match_kernel_variant.argtypes = [ctypes.c_void_p]
-        L.omvg_match_max_clusters.restype = ctypes.c_int
-        L.omvg_match_max_clusters.argtypes = [ctypes.c_void_p]
         _lib = L
     return _lib
 

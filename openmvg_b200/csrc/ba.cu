@@ -65,9 +65,9 @@ struct omvg_ba_ctx {
   DevBuf<unsigned> bitmap, intr_mask; DevBuf<int> wprefix, rowptr, cols;
   DevBuf<double> Scc, Sci, Sii, rhs, Minv_c, Minv_i, work_i;
   DevBuf<double> z, res, pvec, w, zeta, pcg_part;
-  DevBuf<double> gW, gAW, bX, bR, bP, bW, bZ, pcg2_part;   // two-level block-PCG workspaces
+  DevBuf<double> gW, bX, bR, bP, bW, bZ, pcg2_part;   // two-level block-PCG workspaces
   DevBuf<int> agg_of, agg_start, agg_cams, brow, nb_start, nb_list; DevBuf<unsigned short> blk_lcol; int nb_max = 0;   // neighbour lists of the aggregates (pcg5)
-  DevBuf<double> cE, cEinv, cT, cCv, cYv, cCv2, cAW, bP2; int ng = 0, agg_maxsize = 0;
+  DevBuf<double> cE, cT, cCv, cYv, cCv2, cAW, bP2; int ng = 0, agg_maxsize = 0;   // cE: coarse operator, inverted in place
   DevBuf<double> dA, dT;                             // dense reduced system / scratch of its in-place inverse (mid-size scenes)
   DevBuf<double> part, part2, part3, icol_part, scal;
   DevBuf<int> fail;
@@ -200,10 +200,7 @@ int eval_jac(omvg_ba_ctx *c, const omvg_ba_options *o, const Masks &m, int which
   A.obs_w = c->obs_w.p; A.obs_flags = c->obs_flags.p; A.pt_fixed = c->pt_fixed.p;
   if (have_scale) { A.sc_pt = c->sc_pt.p; A.sc_cam = c->sc_cam.p; A.sc_intr = c->sc_intr.p; }
   if (time_it) OMVG_CUDA(cudaEventRecord(c->evj0, c->stream));
-  static const int minb = getenv("OMVG_BA_EVAL_MINB") ? atoi(getenv("OMVG_BA_EVAL_MINB")) : 4;
   if (c->has_ext) eval_kernel<true, 4, true><<<c->eval_grid, EVAL_THREADS, 0, c->stream>>>(A);
-  else if (minb >= 8) eval_kernel<true, 8, false><<<c->eval_grid, EVAL_THREADS, 0, c->stream>>>(A);
-  else if (minb >= 6) eval_kernel<true, 6, false><<<c->eval_grid, EVAL_THREADS, 0, c->stream>>>(A);
   else eval_kernel<true, 4, false><<<c->eval_grid, EVAL_THREADS, 0, c->stream>>>(A);
   LAUNCH_CHECK();
   if (time_it) OMVG_CUDA(cudaEventRecord(c->evj1, c->stream));
@@ -363,8 +360,7 @@ int build_structure(omvg_ba_ctx *c) {
     OMVG_CUDA(cudaStreamSynchronize(c->stream)); }
   const size_t nco_max = (size_t)ng * MAXW;
   if ((rc = c->cE.alloc(nco_max * nco_max))) return rc;
-  if ((rc = c->cEinv.alloc(nco_max * nco_max))) return rc;
-  if ((rc = c->cT.alloc(std::max(nco_max * nco_max, 3 * (size_t)GJ_B * nco_max)))) return rc;   // Cholesky route: T; Gauss-Jordan: Cold/H/Gn
+  if ((rc = c->cT.alloc(3 * (size_t)GJ_B * nco_max))) return rc;   // Gauss-Jordan scratch: Cold / H / Gn
   if ((rc = c->cCv.alloc((size_t)MAXRHS * nco_max))) return rc;
   if ((rc = c->cYv.alloc((size_t)MAXRHS * nco_max))) return rc;
   if ((rc = c->cCv2.alloc((size_t)MAXRHS * nco_max + 1)) || (rc = c->cAW.alloc((size_t)MAXRHS * nco_max + 1))) return rc;
@@ -500,7 +496,7 @@ int omvg_ba_create(omvg_ba_ctx **out, int device, const omvg_ba_problem *P) {
   AL(c->intr_mask, c->ni);
   AL(c->Sci, (size_t)c->ni8 * 6 * c->nc); AL(c->Sii, (size_t)c->ni8 * c->ni8); AL(c->rhs, c->nred); AL(c->Minv_c, 36 * (size_t)c->nc); AL(c->Minv_i, (size_t)c->ni * KI * KI);
   AL(c->work_i, (size_t)c->ni8 * c->ni8 + c->ni8);
-  AL(c->gW, (size_t)MAXW * 6 * c->nc); AL(c->gAW, (size_t)MAXW * 6 * c->nc);
+  AL(c->gW, (size_t)MAXW * 6 * c->nc);
   AL(c->bX, (size_t)MAXRHS * 6 * c->nc); AL(c->bR, (size_t)MAXRHS * 6 * c->nc); AL(c->bP, (size_t)MAXRHS * 6 * c->nc); AL(c->bW, (size_t)MAXRHS * 6 * c->nc); AL(c->bZ, (size_t)MAXRHS * 6 * c->nc);
   AL(c->pcg2_part, (size_t)c->n_sms * PCG2_V);
   AL(c->z, c->nred); AL(c->res, c->nred); AL(c->pvec, c->nred); AL(c->w, c->nred); AL(c->zeta, c->nred); AL(c->pcg_part, 3 * (size_t)c->n_sms * 2);
@@ -579,18 +575,14 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
   int nw = 0;
   if (!use_dense && (rc = make_gauge(c, m, nw))) return rc;
   int n_free_intr = 0; for (unsigned mm : m.intr_mask) n_free_intr += __builtin_popcount(mm);
-  const bool use_pcg2 = n_free_intr <= MAXRHS - 1 && !getenv("OMVG_BA_PCG1");
-  const bool use_pcg3 = use_pcg2 && !getenv("OMVG_BA_PCG2") && c->nc >= 2;
+  // up to 32 free intrinsic columns: block elimination of the intrinsics border (pcg5, else pcg3); otherwise pcg_kernel
+  const bool use_pcg3 = n_free_intr <= MAXRHS - 1 && c->nc >= 2 && !getenv("OMVG_BA_PCG1");
   // the per-observation kernels gather pose records (176 B x n_poses) and points through L1: give them all of it
   OMVG_CUDA(cudaFuncSetAttribute(eval_kernel<true, 4, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
-  OMVG_CUDA(cudaFuncSetAttribute(eval_kernel<true, 6, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
-  OMVG_CUDA(cudaFuncSetAttribute(eval_kernel<true, 8, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
   OMVG_CUDA(cudaFuncSetAttribute(eval_kernel<false, 8, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
   OMVG_CUDA(cudaFuncSetAttribute(eval_kernel<true, 4, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
   OMVG_CUDA(cudaFuncSetAttribute(eval_kernel<false, 8, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0));
-  OMVG_CUDA(cudaFuncSetAttribute(pcg2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Pcg2Smem)));
   OMVG_CUDA(cudaFuncSetAttribute(pcg3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pcg2Smem) + 4 * PCG3_NCO_MAX * sizeof(double))));
-  OMVG_CUDA(cudaFuncSetAttribute(pcg4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pcg2Smem) + 4 * PCG3_NCO_MAX * sizeof(double))));
   if ((rc = read_scalars(c))) return rc;
   account_jac();
   double x_cost = c->h_scal[S_COST];
@@ -604,11 +596,6 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
   long long pcg_total = 0;
   int coarse_age = -1; double last_pcg_its = 0, fresh_pcg_its = 1e30; bool fresh_pending = false;
   static const int coarse_every = getenv("OMVG_BA_COARSE_EVERY") ? std::max(1, atoi(getenv("OMVG_BA_COARSE_EVERY"))) : 3;
-  // Small reduced systems are latency-bound on the grid-wide barriers of the PCG (4-5 us per iteration of pure
-  // synchronisation at 148 CTAs): up to `small_nc` poses ONE CTA runs the whole solve with block barriers instead.
-  // (measured: 0.70 vs 0.74 ms per LM iteration at 10 poses, but 0.99 vs 0.84 at 20: one CTA serialises the SpMV)
-  static const int small_nc = getenv("OMVG_BA_PCG_SMALL") ? atoi(getenv("OMVG_BA_PCG_SMALL")) : 12;
-  const int pcg_grid = (c->nc <= small_nc && use_pcg3) ? 1 : c->n_sms;
   if (!c->gj_grid) {                                        // as many co-resident CTAs as the tile count can use
     int per_sm = 1; OMVG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, coarse_invert_kernel, 256, 0));
     c->gj_grid = c->n_sms * std::max(1, std::min(per_sm, 2));
@@ -625,10 +612,9 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
       const int nb = std::max(1, std::min(2 * c->n_sms, (3 * c->np + 255) / 256));
       lm_diag3_kernel<<<dim3(nb, 3), 256, 0, c->stream>>>(DG, O->min_lm_diagonal, O->max_lm_diagonal, radius); LAUNCH_CHECK(); }
     // ---- reduced camera system
-    const bool split_schur = m.pts_free && !getenv("OMVG_BA_SCHUR1") && !getenv("OMVG_BA_SCHUR2");
-    if (split_schur && !c->corner_rep.p) { if ((rc = c->corner_rep.alloc((size_t)CORNER_REPS * (KI * KI + KI)))) return rc; }
+    if (m.pts_free && !c->corner_rep.p) { if ((rc = c->corner_rep.alloc((size_t)CORNER_REPS * (KI * KI + KI)))) return rc; }
     { Zero4 Z{}; Z.p[0] = c->Scc.p; Z.n[0] = (long long)c->nnzb * 36; Z.p[1] = c->Sci.p; Z.n[1] = (long long)c->Sci.n; Z.p[2] = c->Sii.p; Z.n[2] = (long long)c->Sii.n;
-      Z.p[3] = split_schur ? c->corner_rep.p : c->rhs.p; Z.n[3] = split_schur ? (long long)c->corner_rep.n : 0;     // (rhs is fully written by s_init_kernel)
+      Z.p[3] = m.pts_free ? c->corner_rep.p : c->rhs.p; Z.n[3] = m.pts_free ? (long long)c->corner_rep.n : 0;     // (rhs is fully written by s_init_kernel)
       const int nb = (int)std::max<long long>(1, std::min<long long>(4 * c->n_sms, (Z.n[0] + 255) / 256));
       zero4_kernel<<<dim3(nb, 4), 256, 0, c->stream>>>(Z); LAUNCH_CHECK(); }
     SchurArgs SA{}; SA.r = c->r.p; SA.Jp = c->Jp.p; SA.Jc = c->Jc.p; SA.Ji = c->Ji.p; SA.EtE = c->EtE.p; SA.Etb = c->Etb.p; SA.EtFi = c->EtFi.p; SA.lmD_pt = c->lmD_pt.p; SA.pt_single = c->pt_single.p; SA.FtF = c->FtF.p; SA.FiFi = c->FiFi.p; SA.g_cam = c->g_cam.p; SA.g_intr = c->g_intr.p;
@@ -636,15 +622,11 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
     SA.pts_free = m.pts_free; SA.kiu = c->kiu; SA.bsr = Bsr{c->bitmap.p, c->wprefix.p, c->rowptr.p, c->words}; SA.Scc = c->Scc.p; SA.Sci = c->Sci.p; SA.Sii = c->Sii.p; SA.rhs = c->rhs.p;
     SA.Einv = c->Einv.p; SA.fail = c->fail.p;
     { const int ninit = std::max(std::max(36 * c->nc, 64 * c->ni), c->nred); s_init_kernel<<<(ninit + 255) / 256, 256, 0, c->stream>>>(SA); LAUNCH_CHECK(); }
-    static const bool schur1 = getenv("OMVG_BA_SCHUR1") != nullptr;
     SA.n_points = c->np;
-    static const bool schur2 = getenv("OMVG_BA_SCHUR2") != nullptr;      // fused warp-per-landmark kernel (A/B)
-    if (m.pts_free && !schur1 && !schur2) {
+    if (m.pts_free) {
       if (!c->GE.p) { if ((rc = c->GE.alloc(36 * (size_t)c->no))) return rc; }
       { const unsigned sg = (unsigned)((c->no + SCHUR_THREADS - 1) / SCHUR_THREADS);
-        static const bool minb4 = getenv("OMVG_BA_STAGE_MINB") && atoi(getenv("OMVG_BA_STAGE_MINB")) == 4;   // A/B: 128 registers, 4 CTAs per SM
-#define STAGE(K) do { if (minb4) schur_stage_kernel<K, 4><<<sg, SCHUR_THREADS, 0, c->stream>>>(SA, c->GE.p, c->corner_rep.p); \
-                      else schur_stage_kernel<K, 5><<<sg, SCHUR_THREADS, 0, c->stream>>>(SA, c->GE.p, c->corner_rep.p); } while (0)
+#define STAGE(K) schur_stage_kernel<K><<<sg, SCHUR_THREADS, 0, c->stream>>>(SA, c->GE.p, c->corner_rep.p)
         switch (c->kiu) {        // intrinsic columns in use (as for the column sums)
           case 3: STAGE(3); break;
           case 4: STAGE(4); break;
@@ -659,19 +641,12 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
       static const int occ2 = [] { int o = 1; cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, schur_pair_kernel, 256, 0); return std::max(1, o); }();   // (thread-safe: Adjust may run on several host threads)
       schur_pair_kernel<<<c->n_sms * occ2, 256, 0, c->stream>>>(SA, c->GE.p); LAUNCH_CHECK(); c->launches += 2;
       SA.skip_fast = 1;
-    } else
-    if (m.pts_free && !schur1) {
-      static const int minb = getenv("OMVG_BA_SCHUR2_MINB") ? atoi(getenv("OMVG_BA_SCHUR2_MINB")) : 5;
-      void (*kern)(SchurArgs) = minb >= 6 ? schur_point_kernel<6> : (minb >= 5 ? schur_point_kernel<5> : schur_point_kernel<3>);
-      int occ = 1; OMVG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 32 * SCHUR2_WARPS, 0)); occ = std::max(1, occ);
-      kern<<<c->n_sms * occ, 32 * SCHUR2_WARPS, 0, c->stream>>>(SA); LAUNCH_CHECK(); c->launches++;   // one resident wave, grid-stride over landmarks
-      SA.skip_fast = 1;
     }
-    if (!m.pts_free || schur1 || c->n_slow > 0) { schur_kernel<<<(unsigned)((c->no + SCHUR_THREADS - 1) / SCHUR_THREADS), SCHUR_THREADS, 0, c->stream>>>(SA); LAUNCH_CHECK(); }
+    if (!m.pts_free || c->n_slow > 0) { schur_kernel<<<(unsigned)((c->no + SCHUR_THREADS - 1) / SCHUR_THREADS), SCHUR_THREADS, 0, c->stream>>>(SA); LAUNCH_CHECK(); }
     mirror_kernel<<<(c->nc * 32 + 255) / 256, 256, 0, c->stream>>>(c->Scc.p, SA.bsr, c->cols.p, c->nc); LAUNCH_CHECK();
     c->launches += 2;
     finish_cam_kernel<<<(c->nc + 63) / 64, 64, 0, c->stream>>>(c->Scc.p, SA.bsr, c->lmD_cam.p, m.pose_mask, c->nc, c->Minv_c.p, c->fail.p, use_dense ? 0 : 1); LAUNCH_CHECK();
-    finish_intr_kernel<<<1, 256, 0, c->stream>>>(c->Sii.p, c->lmD_intr.p, c->intr_mask.p, c->ni8, c->Minv_i.p, c->work_i.p, c->fail.p, (use_pcg2 || use_dense) ? 0 : 1); LAUNCH_CHECK();
+    finish_intr_kernel<<<1, 256, 0, c->stream>>>(c->Sii.p, c->lmD_intr.p, c->intr_mask.p, c->ni8, c->Minv_i.p, c->work_i.p, c->fail.p, (use_pcg3 || use_dense) ? 0 : 1); LAUNCH_CHECK();
     // ---- PCG on S z = rhs
     PcgArgs PA{}; PA.Scc = c->Scc.p; PA.rowptr = c->rowptr.p; PA.cols = c->cols.p; PA.Sci = c->Sci.p; PA.Sii = c->Sii.p; PA.rhs = c->rhs.p; PA.Minv_c = c->Minv_c.p; PA.Minv_i = c->Minv_i.p;
     PA.n_poses = c->nc; PA.ni8 = c->ni8; PA.z = c->z.p; PA.res = c->res.p; PA.p = c->pvec.p; PA.w = c->w.p; PA.zeta = c->zeta.p; PA.part = c->pcg_part.p;
@@ -681,9 +656,8 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
     // iterations (measured 38->40, 42->49, 43->43) but saves its O(nco^3) setup, so it is refreshed every
     // `coarse_every` LM steps (measured at 1000 cameras, ms per solve: every step 17.9, 2: 16.0, 3: 15.2, 5: 15.9),
     // or earlier if the last solve needed 1.5x the iterations seen right after a refresh.
-    const bool use_coarse = !use_dense && (use_pcg3 || !use_pcg2) && nw > 0 && c->nc >= 2;
+    const bool use_coarse = !use_dense && nw > 0 && c->nc >= 2;
     const Coarse CO{c->agg_of.p, c->agg_start.p, c->agg_cams.p, c->ng, nw, use_coarse ? c->ng * nw : 0};
-    static const bool use_chol = getenv("OMVG_BA_COARSE_CHOL") != nullptr;
     if (use_coarse) {
       const int nco = CO.nco;
       const bool refresh = nco > 0 && (coarse_age < 0 || coarse_age >= coarse_every || last_pcg_its > 1.5 * fresh_pcg_its + 5);
@@ -692,27 +666,20 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
       if (refresh) {
         OMVG_CUDA(cudaMemsetAsync(c->cE.p, 0, (size_t)nco * nco * sizeof(double), c->stream));
         coarse_assemble_kernel<<<(c->nnzb + 127) / 128, 128, 0, c->stream>>>(c->Scc.p, c->brow.p, c->cols.p, c->nnzb, c->gW.p, c->nc, CO, c->cE.p); LAUNCH_CHECK();
-        if (!use_chol) {                                        // blocked Gauss-Jordan, in place: cE becomes E^-1
-          double *Ep = c->cE.p, *Tp = c->cT.p; int nn = nco; int *fp = c->fail.p;
-          static const bool gj_timing = getenv("OMVG_BA_GJ_TIMING") != nullptr;
-          unsigned long long *tp = nullptr;
-          if (gj_timing) { if (!c->pcg_tim.p) { if ((rc = c->pcg_tim.alloc(8))) return rc; } OMVG_CUDA(cudaMemsetAsync(c->pcg_tim.p, 0, 64, c->stream)); tp = c->pcg_tim.p; }
-          void *cargs[] = {&Ep, &nn, &Tp, &fp, &tp};
-          const int mt = (nco + CT - 1) / CT;                   // no more CTAs than 64x64 tiles: a small coarse space pays for fewer barrier participants
-          const int gj = std::max(1, std::min(c->gj_grid, mt * mt));
-          OMVG_CUDA(cudaLaunchCooperativeKernel((void *)coarse_invert_kernel, dim3(gj), dim3(256), cargs, 0, c->stream));
-          if (gj_timing) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
-            fprintf(stderr, "[omvg_ba gj timing] us: pivot inverse %.1f slices %.1f sync %.1f tiles %.1f sync %.1f (n %d, %d CTAs)\n", h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3, h[3] * 1e-3, h[4] * 1e-3, nco, c->gj_grid); }
-        } else {
-          const size_t sm = sizeof(double) * ((size_t)CNB * CNB + 2 * CT * (CNB + 1) + 2 * CT * (CT + 1));
-          OMVG_CUDA(cudaFuncSetAttribute(coarse_setup_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-          double *Ep = c->cE.p, *Tp = c->cT.p, *Ip = c->cEinv.p; int nn = nco; int *fp = c->fail.p;
-          void *cargs[] = {&Ep, &nn, &Tp, &Ip, &fp};
-          OMVG_CUDA(cudaLaunchCooperativeKernel((void *)coarse_setup_kernel, dim3(pcg_grid), dim3(256), cargs, sm, c->stream)); }
+        // blocked Gauss-Jordan, in place: cE becomes E^-1
+        double *Ep = c->cE.p, *Tp = c->cT.p; int nn = nco; int *fp = c->fail.p;
+        static const bool gj_timing = getenv("OMVG_BA_GJ_TIMING") != nullptr;
+        unsigned long long *tp = nullptr;
+        if (gj_timing) { if (!c->pcg_tim.p) { if ((rc = c->pcg_tim.alloc(8))) return rc; } OMVG_CUDA(cudaMemsetAsync(c->pcg_tim.p, 0, 64, c->stream)); tp = c->pcg_tim.p; }
+        void *cargs[] = {&Ep, &nn, &Tp, &fp, &tp};
+        const int mt = (nco + CT - 1) / CT;                   // no more CTAs than 64x64 tiles: a small coarse space pays for fewer barrier participants
+        const int gj = std::max(1, std::min(c->gj_grid, mt * mt));
+        OMVG_CUDA(cudaLaunchCooperativeKernel((void *)coarse_invert_kernel, dim3(gj), dim3(256), cargs, 0, c->stream));
+        if (gj_timing) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
+          fprintf(stderr, "[omvg_ba gj timing] us: pivot inverse %.1f slices %.1f sync %.1f tiles %.1f sync %.1f (n %d, %d CTAs)\n", h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3, h[3] * 1e-3, h[4] * 1e-3, nco, c->gj_grid); }
         c->launches += 2;
       }
     }
-    const double *Einv_p = use_chol ? c->cEinv.p : c->cE.p;
     if (use_dense2) {
       int nd = 6 * c->nc + c->ni8;
       if (!c->dA.p) { if ((rc = c->dA.alloc((size_t)nd * nd)) || (rc = c->dT.alloc(3 * (size_t)GJ_B * nd))) return rc; }
@@ -736,61 +703,43 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
       if (dense_timing) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
         fprintf(stderr, "[omvg_ba dense timing] n %d us: assemble %.1f factor %.1f backward %.1f\n", nd, h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3); }
     } else
-    if (use_pcg2) {
+    if (use_pcg3) {
       Pcg2Args P2{}; P2.Scc = c->Scc.p; P2.rowptr = c->rowptr.p; P2.cols = c->cols.p; P2.Sci = c->Sci.p; P2.Sii = c->Sii.p; P2.rhs = c->rhs.p; P2.Minv_c = c->Minv_c.p;
       P2.W = c->gW.p; P2.intr_mask = c->intr_mask.p; P2.n_poses = c->nc; P2.ni8 = c->ni8; P2.nw = nw; P2.X = c->bX.p; P2.Rv = c->bR.p; P2.Pv = c->bP.p; P2.Wv = c->bW.p; P2.Zv = c->bZ.p;
-      P2.AW = c->gAW.p; P2.part = c->pcg2_part.p; P2.z = c->z.p; P2.tol = O->pcg_tolerance; P2.max_iter = O->pcg_max_iterations; P2.out = c->scal.p + S_PCG_IT;
-      if (use_pcg3) {
-        Pcg3Args P3{}; P3.base = P2; P3.C = CO; P3.C.nco = c->ng * nw; P3.Einv = Einv_p; P3.Cv = c->cCv.p; P3.Yv = c->cYv.p; P3.Pv2 = c->bP2.p;
-        static const bool pcg_timing = getenv("OMVG_BA_PCG_TIMING") != nullptr;
-        if (pcg_timing) { if (!c->pcg_tim.p) { if ((rc = c->pcg_tim.alloc(8))) return rc; } OMVG_CUDA(cudaMemsetAsync(c->pcg_tim.p, 0, 64, c->stream)); P3.tim = c->pcg_tim.p; }
-        // pcg4 (2 grid syncs per iteration instead of 4) is kept for A/B and for the single-CTA mode: at 148 CTAs it is
-        // NOT faster (measured, config 2: 14.7 vs 14.2 ms per solve) — every CTA re-stages the whole coarse residual
-        // (6 us per iteration) where v3 pays its two extra barriers (2 x 3.5 us).  See DESIGN.md §4.3.
-        // v5: shared-memory resident, aggregate-owned (2 barriers + 2 L2 round trips per iteration).  Needs one CTA per
-        // aggregate, <= 4 right-hand sides (1 + free intrinsic columns) and aggregates of <= 16 cameras; else v3.
-        static const bool no_pcg5 = getenv("OMVG_BA_PCG3") != nullptr || getenv("OMVG_BA_PCG4") != nullptr;
-        const int nrhs_host = 1 + n_free_intr;
-        if (!no_pcg5 && pcg_grid > 1 && nrhs_host <= PCG5_NR && c->ng <= pcg_grid && c->agg_maxsize <= PCG5_MC && c->nb_max <= PCG5_NB && P3.C.nco <= PCG3_NCO_MAX) {
-          const size_t fixed = sizeof(Pcg5Red) + sizeof(Pcg5Smem) + (size_t)PCG5_NR * PCG3_NCO_MAX * sizeof(double) + (size_t)PCG5_NB * PCG5_PS * sizeof(double);
-          static const int smem_max = [] { int v = 0, dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev); return v; }();
-          const int nb_cache = (int)std::max<long long>(0, ((long long)smem_max - (long long)fixed - 2048) /   /* (static shared memory of the kernel + slack) */ (long long)(PCG5_BS * sizeof(double) + sizeof(unsigned short)));
-          const size_t smem = fixed + (size_t)nb_cache * (PCG5_BS * sizeof(double) + sizeof(unsigned short)) + 16;
-          OMVG_CUDA(cudaFuncSetAttribute(pcg5_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-          double *cg2 = c->cCv2.p, *aw = c->cAW.p; int nbc = nb_cache; const int *nbs = c->nb_start.p, *nbl = c->nb_list.p; const unsigned short *lc = c->blk_lcol.p;
-          void *args[] = {&P3, &cg2, &aw, &nbc, &nbs, &nbl, &lc};
-          // one CTA per aggregate and no more: idle CTAs would only add participants to the two barriers of every iteration
-          OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg5_kernel, dim3(std::max(1, c->ng)), dim3(PCG2_THREADS), args, smem, c->stream));
-          if (pcg_timing) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
-            fprintf(stderr, "[omvg_ba pcg5 timing] us: A wait-AW %.1f y %.1f local %.1f reduce %.1f | B gather %.1f rows %.1f publish %.1f reduce %.1f (cache %d blocks)\n", h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3, h[3] * 1e-3, h[6] * 1e-3, h[7] * 1e-3, h[4] * 1e-3, h[5] * 1e-3, nb_cache); P3.tim = nullptr; }
-        } else {
-        static const bool want_pcg4 = getenv("OMVG_BA_PCG4") != nullptr;
-        if ((want_pcg4 || pcg_grid == 1) && P3.C.nco <= PCG3_NCO_MAX) {
-          double *cv2 = c->cCv2.p, *aw = c->cAW.p;
-          void *args[] = {&P3, &cv2, &aw};
-          OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg4_kernel, dim3(pcg_grid), dim3(PCG2_THREADS), args, sizeof(Pcg2Smem) + 4 * PCG3_NCO_MAX * sizeof(double), c->stream));
-          if (pcg_timing) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
-            fprintf(stderr, "[omvg_ba pcg4 timing] us: A stage %.1f y %.1f update+z %.1f reduce %.1f | B spmv %.1f reduce %.1f\n", h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3, h[3] * 1e-3, h[4] * 1e-3, h[5] * 1e-3); P3.tim = nullptr; }
-        } else {
-        void *args[] = {&P3};
-        OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg3_kernel, dim3(pcg_grid), dim3(PCG2_THREADS), args, sizeof(Pcg2Smem) + 4 * PCG3_NCO_MAX * sizeof(double), c->stream));
-        }
-        }
-        if (pcg_timing && P3.tim) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
-          fprintf(stderr, "[omvg_ba pcg timing] us: coarse (stage %.1f rows %.1f sync %.1f) z %.1f spmv %.1f update %.1f tail %.1f border %.1f\n", h[6] * 1e-3, h[7] * 1e-3, h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3, h[3] * 1e-3, h[4] * 1e-3, h[5] * 1e-3); }
+      P2.part = c->pcg2_part.p; P2.z = c->z.p; P2.tol = O->pcg_tolerance; P2.max_iter = O->pcg_max_iterations; P2.out = c->scal.p + S_PCG_IT;
+      Pcg3Args P3{}; P3.base = P2; P3.C = CO; P3.C.nco = c->ng * nw; P3.Einv = c->cE.p; P3.Cv = c->cCv.p; P3.Yv = c->cYv.p; P3.Pv2 = c->bP2.p;
+      static const bool pcg_timing = getenv("OMVG_BA_PCG_TIMING") != nullptr;
+      if (pcg_timing) { if (!c->pcg_tim.p) { if ((rc = c->pcg_tim.alloc(8))) return rc; } OMVG_CUDA(cudaMemsetAsync(c->pcg_tim.p, 0, 64, c->stream)); P3.tim = c->pcg_tim.p; }
+      // pcg5: shared-memory resident, aggregate-owned (2 barriers + 2 L2 round trips per iteration).  Needs one CTA per
+      // aggregate, <= 4 right-hand sides (1 + free intrinsic columns) and aggregates of <= 16 cameras; else pcg3.
+      const int nrhs_host = 1 + n_free_intr;
+      if (nrhs_host <= PCG5_NR && c->ng <= c->n_sms && c->agg_maxsize <= PCG5_MC && c->nb_max <= PCG5_NB && P3.C.nco <= PCG3_NCO_MAX) {
+        const size_t fixed = sizeof(Pcg5Red) + sizeof(Pcg5Smem) + (size_t)PCG5_NR * PCG3_NCO_MAX * sizeof(double) + (size_t)PCG5_NB * PCG5_PS * sizeof(double);
+        static const int smem_max = [] { int v = 0, dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev); return v; }();
+        const int nb_cache = (int)std::max<long long>(0, ((long long)smem_max - (long long)fixed - 2048) /   /* (static shared memory of the kernel + slack) */ (long long)(PCG5_BS * sizeof(double) + sizeof(unsigned short)));
+        const size_t smem = fixed + (size_t)nb_cache * (PCG5_BS * sizeof(double) + sizeof(unsigned short)) + 16;
+        OMVG_CUDA(cudaFuncSetAttribute(pcg5_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        double *cg2 = c->cCv2.p, *aw = c->cAW.p; int nbc = nb_cache; const int *nbs = c->nb_start.p, *nbl = c->nb_list.p; const unsigned short *lc = c->blk_lcol.p;
+        void *args[] = {&P3, &cg2, &aw, &nbc, &nbs, &nbl, &lc};
+        // one CTA per aggregate and no more: idle CTAs would only add participants to the two barriers of every iteration
+        OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg5_kernel, dim3(std::max(1, c->ng)), dim3(PCG2_THREADS), args, smem, c->stream));
+        if (pcg_timing) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
+          fprintf(stderr, "[omvg_ba pcg5 timing] us: A wait-AW %.1f y %.1f local %.1f reduce %.1f | B gather %.1f rows %.1f publish %.1f reduce %.1f (cache %d blocks)\n", h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3, h[3] * 1e-3, h[6] * 1e-3, h[7] * 1e-3, h[4] * 1e-3, h[5] * 1e-3, nb_cache); }
       } else {
-        void *args[] = {&P2};
-        OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg2_kernel, dim3(pcg_grid), dim3(PCG2_THREADS), args, sizeof(Pcg2Smem), c->stream));
+        void *args[] = {&P3};
+        OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg3_kernel, dim3(c->n_sms), dim3(PCG2_THREADS), args, sizeof(Pcg2Smem) + 4 * PCG3_NCO_MAX * sizeof(double), c->stream));
+        if (pcg_timing) { unsigned long long h[8]; OMVG_CUDA(cudaMemcpyAsync(h, c->pcg_tim.p, 64, cudaMemcpyDeviceToHost, c->stream)); OMVG_CUDA(cudaStreamSynchronize(c->stream));
+          fprintf(stderr, "[omvg_ba pcg timing] us: coarse (stage %.1f rows %.1f sync %.1f) z %.1f spmv %.1f update %.1f tail %.1f border %.1f\n", h[6] * 1e-3, h[7] * 1e-3, h[0] * 1e-3, h[1] * 1e-3, h[2] * 1e-3, h[3] * 1e-3, h[4] * 1e-3, h[5] * 1e-3); }
       }
     } else {
-      // more than 32 free intrinsic columns (e.g. one intrinsic group per image): PCG on the whole reduced system
-      // [Scc Sci'; Sci Sii] with the same aggregated coarse space on the camera rows and block-Jacobi on the intrinsics
-      if (use_coarse) { PA.W = c->gW.p; PA.C = CO; PA.Einv = Einv_p; PA.Cv = c->cCv.p; PA.Yv = c->cYv.p; }
-      void *args[] = {&PA}; OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg_kernel, dim3(pcg_grid), dim3(256), args, 0, c->stream));
+      // more than 32 free intrinsic columns (e.g. one intrinsic group per image), a single pose, or OMVG_BA_PCG1: PCG on the
+      // whole reduced system [Scc Sci'; Sci Sii] with the aggregated coarse space on the camera rows (when there is one) and
+      // block-Jacobi on the intrinsics
+      if (use_coarse) { PA.W = c->gW.p; PA.C = CO; PA.Einv = c->cE.p; PA.Cv = c->cCv.p; PA.Yv = c->cYv.p; }
+      void *args[] = {&PA}; OMVG_CUDA(cudaLaunchCooperativeKernel((void *)pcg_kernel, dim3(c->n_sms), dim3(256), args, 0, c->stream));
     }
     // ---- back substitution, step = -y
-    static const bool backsub1 = getenv("OMVG_BA_BACKSUB1") != nullptr;
-    if (backsub1 || !m.pts_free) {
+    if (!m.pts_free) {
       backsub_kernel<<<(c->np + 127) / 128, 128, 0, c->stream>>>(c->Jp.p, c->Jc.p, c->Ji.p, c->Etb.p, c->Einv.p, c->obs_pose.p, c->obs_intr.p, c->pt_start.p, c->np, c->nc, c->no, c->kiu,
                                                                c->z.p, m.pts_free, c->step_pt.p); LAUNCH_CHECK();
     } else {

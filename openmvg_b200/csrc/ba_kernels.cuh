@@ -662,8 +662,8 @@ struct SchurArgs {
   const int *obs_pose, *obs_intr, *obs_pt, *pt_start; const unsigned char *pt_single;
   const double *FtF, *FiFi, *g_cam, *g_intr;
   long long n; int n_poses, n_intr, pts_free, kiu;
-  int n_points;     // schur_point_kernel: landmarks
-  int skip_fast;    // schur_kernel: leave the landmarks schur_point_kernel handles (pt_single and <= 32 observations) alone
+  int n_points;     // schur_pair_kernel: landmarks
+  int skip_fast;    // schur_kernel: leave the landmarks the split Schur step handles (pt_single and <= 32 observations) alone
   Bsr bsr;
   double *Scc;      // [nnzb][36]
   double *Sci;      // [KI*n_intr][6*n_poses]
@@ -827,139 +827,23 @@ __global__ void __launch_bounds__(SCHUR_THREADS) schur_kernel(SchurArgs A) {
   }
 }
 
-// lower triangle of Scc from the upper one: block (a,b), a > b, = block (b,a)'
-// One WARP per landmark (the common case: all its observations through one intrinsic group, at most 32 of
-// them).  Lane l stages Einv E'Fc and E'Fc of observation l in shared memory and does the per-observation
-// border / right-hand-side terms; then the warp walks the camera pairs (cam(u) >= cam(t)) TOGETHER, lane e
-// adding element e of the 6x6 block: one RED instruction touches the 9 sectors of one block instead of 32
-// sectors of 32 different blocks.  Measured on B200 (tools/atomic_bench.cu): 565 vs 222 G FP64 atomics/s.
-constexpr int SCHUR2_WARPS = 4;
 constexpr int CORNER_REPS = 64;
-template <int MINB>
-__global__ void __launch_bounds__(32 * SCHUR2_WARPS, MINB) schur_point_kernel(SchurArgs A) {
-  __shared__ double s_gt[SCHUR2_WARPS][32][18];
-  __shared__ double s_ef[SCHUR2_WARPS][32][18];
-  __shared__ int s_cam[SCHUR2_WARPS][32];
-  __shared__ double s_ii[KI * KI + KI];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int gwarp = blockIdx.x * SCHUR2_WARPS + wib, nwarps = gridDim.x * SCHUR2_WARPS;
-  const long long n = A.n;
-  const int nred_c = 6 * A.n_poses, ni8 = KI * A.n_intr;
-  if (threadIdx.x < KI * KI + KI) s_ii[threadIdx.x] = 0.0;
-  __syncthreads();
-  const int q0 = A.obs_intr[0];                               // the corner of this group is reduced per CTA in shared memory
-  for (int j = gwarp; j < A.n_points; j += nwarps) {
-    const int t0 = A.pt_start[j], K = A.pt_start[j + 1] - t0;
-    if (K == 0 || K > 32 || !A.pt_single[j]) continue;         // schur_kernel (skip_fast) takes the others
-    double inv[9], ie[3], m[6];
-    { const double *E = A.EtE + 6 * (size_t)j;
-      const double d0 = A.lmD_pt[3 * j], d1 = A.lmD_pt[3 * j + 1], d2 = A.lmD_pt[3 * j + 2];
-      m[0] = E[0] + d0 * d0; m[1] = E[1]; m[2] = E[2] + d1 * d1; m[3] = E[3]; m[4] = E[4]; m[5] = E[5] + d2 * d2; }
-    if (!inv3_spd(m, inv)) { if (lane == 0) atomicExch(A.fail, 1); }
-    { const double *eb = A.Etb + 3 * (size_t)j;
-      #pragma unroll
-      for (int a = 0; a < 3; ++a) ie[a] = inv[a * 3] * eb[0] + inv[a * 3 + 1] * eb[1] + inv[a * 3 + 2] * eb[2]; }
-    if (lane < 9) A.Einv[9 * (size_t)j + lane] = inv[lane];
-    __syncwarp();
-    if (lane < K) {
-      const long long t = t0 + lane;
-      const int ct = A.obs_pose[t], qt = A.obs_intr[t];
-      double jc[12], ji[2 * KI], jp[6];
-      #pragma unroll
-      for (int k = 0; k < 12; ++k) jc[k] = A.Jc[k * n + t];
-      #pragma unroll
-      for (int k = 0; k < 2 * KI; ++k) ji[k] = (k % KI) < A.kiu ? A.Ji[k * n + t] : 0.0;
-      #pragma unroll
-      for (int k = 0; k < 6; ++k) jp[k] = A.Jp[k * n + t];
-      double efc[18];                                          // E'Fc of this observation (3x6)
-      #pragma unroll
-      for (int a = 0; a < 3; ++a)
-        #pragma unroll
-        for (int c = 0; c < 6; ++c) efc[a * 6 + c] = jp[a] * jc[c] + jp[3 + a] * jc[6 + c];
-      #pragma unroll
-      for (int c = 0; c < 6; ++c) atomicAdd(&A.rhs[6 * ct + c], -(efc[c] * ie[0] + efc[6 + c] * ie[1] + efc[12 + c] * ie[2]));
-      // border with the point-summed E'Fi:  Sci(qt; ct) += Fi'Fc - (Einv E'Fi_pt)' E'Fc
-      double *sci_row0 = A.Sci + (size_t)(KI * qt) * nred_c + 6 * ct;
-      const double *fi = A.EtFi + (size_t)j * 3 * KI;
-      #pragma unroll
-      for (int a = 0; a < KI; ++a) {
-        const double f0 = fi[a], f1 = fi[KI + a], f2 = fi[2 * KI + a];
-        if (f0 == 0.0 && f1 == 0.0 && f2 == 0.0 && ji[a] == 0.0 && ji[KI + a] == 0.0) continue;   // constant parameter
-        const double g0 = inv[0] * f0 + inv[1] * f1 + inv[2] * f2, g1 = inv[3] * f0 + inv[4] * f1 + inv[5] * f2, g2 = inv[6] * f0 + inv[7] * f1 + inv[8] * f2;
-        #pragma unroll
-        for (int b = 0; b < 6; ++b)
-          atomicAdd(&sci_row0[(size_t)a * nred_c + b], ji[a] * jc[b] + ji[KI + a] * jc[6 + b] - (g0 * efc[b] + g1 * efc[6 + b] + g2 * efc[12 + b]));
-        if (lane == 0) {                                        // once per point: corner and its right-hand side
-          const double rv = -(f0 * ie[0] + f1 * ie[1] + f2 * ie[2]);
-          if (qt == q0) atomicAdd(&s_ii[KI * KI + a], rv); else atomicAdd(&A.rhs[nred_c + KI * qt + a], rv);
-          #pragma unroll
-          for (int b = 0; b < KI; ++b) {
-            const double v = -(g0 * fi[b] + g1 * fi[KI + b] + g2 * fi[2 * KI + b]);
-            if (v == 0.0) continue;
-            if (qt == q0) atomicAdd(&s_ii[a * KI + b], v); else atomicAdd(&A.Sii[(size_t)(KI * qt + a) * ni8 + KI * qt + b], v);
-          }
-        }
-      }
-      #pragma unroll
-      for (int a = 0; a < 3; ++a)
-        #pragma unroll
-        for (int c = 0; c < 6; ++c) {
-          s_ef[wib][lane][a * 6 + c] = efc[a * 6 + c];
-          s_gt[wib][lane][a * 6 + c] = inv[a * 3] * efc[c] + inv[a * 3 + 1] * efc[6 + c] + inv[a * 3 + 2] * efc[12 + c];   // Einv * E'Fc_t
-        }
-      s_cam[wib][lane] = ct;
-    }
-    __syncwarp();
-    // camera pairs: Scc(ct, cu) -= (Einv E'Fc_t)' E'Fc_u  for cam(u) >= cam(t)
-    const int ea = lane / 6, eb2 = lane % 6, fa = (32 + lane) / 6, fb = (32 + lane) % 6;   // element lane, and 32 + lane (lanes 0..3)
-    // block index of (cam(tt), cam(lane)): looked up by all lanes at once, one row ahead of its use, so the
-    // dependent bitmap loads never sit between two atomics
-    // block index of (cam(tt), cam(lane)): the three bitmap-BSR words are LOADED one row ahead (before the
-    // atomics of the current row) and only combined after them, so their latency hides behind the inner loop
-    const int cam_l = lane < K ? s_cam[wib][lane] : 0;
-    const unsigned lowmask = (1u << (cam_l & 31)) - 1u;
-    int rp = 0, wp = 0; unsigned bm = 0;
-    { const int c0 = s_cam[wib][0]; const size_t w = (size_t)c0 * A.bsr.words + (cam_l >> 5); rp = A.bsr.rowptr[c0]; wp = A.bsr.wprefix[w]; bm = A.bsr.bitmap[w]; }
-    for (int tt = 0; tt < K; ++tt) {
-      const int ctt = s_cam[wib][tt];
-      const int cur = (lane < K && cam_l >= ctt) ? rp + wp + __popc(bm & lowmask) : -1;
-      if (tt + 1 < K) { const int cn = s_cam[wib][tt + 1]; const size_t w = (size_t)cn * A.bsr.words + (cam_l >> 5); rp = A.bsr.rowptr[cn]; wp = A.bsr.wprefix[w]; bm = A.bsr.bitmap[w]; }
-      const double g0 = s_gt[wib][tt][ea], g1 = s_gt[wib][tt][6 + ea], g2 = s_gt[wib][tt][12 + ea];
-      const double h0 = lane < 4 ? s_gt[wib][tt][fa] : 0.0, h1 = lane < 4 ? s_gt[wib][tt][6 + fa] : 0.0, h2 = lane < 4 ? s_gt[wib][tt][12 + fa] : 0.0;
-      unsigned todo = __ballot_sync(0xffffffffu, cur >= 0);
-      while (todo) {
-        const int u = __ffs(todo) - 1; todo &= todo - 1;
-        const int bi = __shfl_sync(0xffffffffu, cur, u);
-        double *blk = A.Scc + 36 * (size_t)bi;
-        const double *ef = s_ef[wib][u];
-        atomicAdd(blk + lane, -(g0 * ef[eb2] + g1 * ef[6 + eb2] + g2 * ef[12 + eb2]));
-        if (lane < 4) atomicAdd(blk + 32 + lane, -(h0 * ef[fb] + h1 * ef[6 + fb] + h2 * ef[12 + fb]));
-      }
-    }
-    __syncwarp();
-  }
-  __syncthreads();
-  if (threadIdx.x < KI * KI + KI) {
-    const double v = s_ii[threadIdx.x];
-    if (v != 0.0) {
-      if (threadIdx.x < KI * KI) atomicAdd(&A.Sii[(size_t)(KI * q0 + threadIdx.x / KI) * ni8 + KI * q0 + threadIdx.x % KI], v);
-      else atomicAdd(&A.rhs[nred_c + KI * q0 + (threadIdx.x - KI * KI)], v);
-    }
-  }
-}
 
-// ---- split form of the warp-per-landmark Schur step (default): the staging half needs ~160 registers, the pair
-// walk ~40; in one kernel the walk ran at 12-20 warps per SM and was latency-bound (0.94 ms).  Here
+// ---- warp-per-landmark Schur step for the common landmark (all its observations through one intrinsic group, at most
+// 32 of them), in two kernels: the staging half needs ~160 registers, the pair walk ~40; fused into one kernel the walk
+// ran at 12-20 warps per SM and was latency-bound (0.94 ms).
 //   schur_stage_kernel : thread per observation (coalesced component-major loads), per-observation border / rhs
 //                        terms, writes GE[obs] = { Einv E'Fc (18), E'Fc (18) }  (288 B per observation)
-//   schur_pair_kernel  : warp per landmark, lane e adds element e of block (cam_t, cam_u) reading GE through L1
+//   schur_pair_kernel  : warp per landmark, lane e adds element e of block (cam_t, cam_u) reading GE through L1: one RED
+//                        instruction touches the 9 sectors of one block instead of 32 sectors of 32 different blocks
+//                        (measured on B200, tools/atomic_bench.cu: 565 vs 222 G FP64 atomics/s)
 // KIU = intrinsic columns in use (3 pinhole .. 8 Brown): the generic 8-column body kept 16 Jacobian and 24 EtFi values
 // live per thread (162 registers, 3 CTAs per SM, 17 % of the warps active, 5x off its DRAM time).  The 36 doubles of an
 // observation's {E^-1 E'F, E'F} record go through shared memory so that a warp writes its 32 records (9 KB, contiguous)
 // with full 256-byte stores instead of 36 scattered 8-byte stores per lane.
 constexpr int GE_LD = 37;                            // padded record stride in shared memory (conflict-free for both phases)
-template <int KIU, int MINB>
-__global__ void __launch_bounds__(SCHUR_THREADS, MINB) schur_stage_kernel(SchurArgs A, double *__restrict__ GE, double *__restrict__ corner_rep) {
+template <int KIU>
+__global__ void __launch_bounds__(SCHUR_THREADS, 5) schur_stage_kernel(SchurArgs A, double *__restrict__ GE, double *__restrict__ corner_rep) {
   // The intrinsics corner (and its rhs) of group q0 is hit once per landmark: accumulate into CORNER_REPS replicas
   // with native FP64 REDs (shared-memory double atomics are CAS loops: they cost 0.3 ms here) and fold them after.
   __shared__ double ge_s[SCHUR_THREADS / 32][32 * GE_LD];
@@ -1096,6 +980,7 @@ __global__ void __launch_bounds__(256) schur_pair_kernel(SchurArgs A, const doub
   }
 }
 
+// lower triangle of Scc from the upper one: block (a,b), a > b, = block (b,a)'
 __global__ void mirror_kernel(double *__restrict__ Scc, Bsr B, const int *__restrict__ cols, int n_poses) {
   const int a = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (a >= n_poses) return;
@@ -1423,7 +1308,7 @@ __global__ void __launch_bounds__(256) pcg_kernel(PcgArgs A) {
   if (tid == 0) { A.out[0] = (double)(it > A.max_iter ? A.max_iter : it); A.out[1] = bnorm2 > 0 ? sqrt(rr / bnorm2) : 0.0; A.out[2] = sqrt(bnorm2); }
 }
 
-// ------------------------------------------------------------------------------ PCG v2
+// ------------------------------------------------------------------------------ block-PCG (pcg3 / pcg5): common parts
 // Two-level preconditioned block-PCG on the camera-camera part of the reduced system, with the
 // (small, dense) intrinsics border removed by block elimination:
 //     [Scc Sci'] [zc]   [bc]        Scc Y = [bc | Sci'] (1 + ni8 right-hand sides, solved together)
@@ -1485,7 +1370,7 @@ struct Pcg2Args {
   const unsigned *intr_mask;  // free intrinsic parameters (block elimination columns)
   int n_poses, ni8, nw;
   double *X, *Rv, *Pv, *Wv, *Zv;   // [nrhs][nc6] each
-  double *AW;                 // [nw][nc6]
+  double *AW;                 // not read by pcg3 / pcg5 (left null); kept so that their parameter layout, and code, stay as measured
   double *part;               // [gridDim.x][PCG2_V] partial reductions
   double *z;                  // out: reduced step [nc6 + ni8]
   double tol; int max_iter;
@@ -1521,7 +1406,7 @@ template <class SM> __device__ __forceinline__ void vsum_begin(SM &S, int V) {
 // fixed butterfly — the same order in every block, hence bitwise identical totals everywhere.
 template <class SM> __device__ __forceinline__ void vsum_end(cg::grid_group &grid, SM &S, int V, double *part) {
   __syncthreads();
-  if (gridDim.x == 1) {                      // single-CTA solve (small problems): a block barrier is the grid barrier
+  if (gridDim.x == 1) {                      // single-CTA solve (pcg5 with one aggregate): a block barrier is the grid barrier
     for (int i = threadIdx.x; i < V; i += PCG2_THREADS) { double t = 0; for (int w = 0; w < PCG2_THREADS / 32; ++w) t += S.wpart[w][i]; S.tot[i] = t; }
     __threadfence_block();
     __syncthreads();
@@ -1540,204 +1425,8 @@ template <class SM> __device__ __forceinline__ void vsum_end(cg::grid_group &gri
   __syncthreads();
 }
 
-// Y[j] = Scc X[j] for j < nv (every S block is read once per group of 3 vectors).  If dot_base >= 0,
-// lane 0 also accumulates X[j].Y[j] over its rows into this warp's slot dot_base + j.
-__device__ __forceinline__ void spmv_multi(const Pcg2Args &A, Pcg2Smem &S, const double *__restrict__ X, double *__restrict__ Y, int nv,
-                                           const unsigned char *skip, int dot_base) {
-  const int lane = threadIdx.x & 31, warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
-  const size_t nc6 = 6 * (size_t)A.n_poses;
-  for (int a = warp; a < A.n_poses; a += nwarps) {
-    for (int j0 = 0; j0 < nv; j0 += 3) {
-      double acc[3][6];
-      #pragma unroll
-      for (int j = 0; j < 3; ++j)
-        #pragma unroll
-        for (int i = 0; i < 6; ++i) acc[j][i] = 0.0;
-      for (int e = A.rowptr[a] + lane; e < A.rowptr[a + 1]; e += 32) {
-        const double *blk = A.Scc + 36 * (size_t)e; const int cb = 6 * A.cols[e];
-        double b[36];
-        #pragma unroll
-        for (int i = 0; i < 36; ++i) b[i] = blk[i];
-        #pragma unroll
-        for (int j = 0; j < 3; ++j) {
-          if (j0 + j < nv && !(skip && skip[j0 + j])) {
-            const double *xb = X + (size_t)(j0 + j) * nc6 + cb;
-            double xv[6];
-            #pragma unroll
-            for (int k = 0; k < 6; ++k) xv[k] = xb[k];
-            #pragma unroll
-            for (int i = 0; i < 6; ++i)
-              #pragma unroll
-              for (int k = 0; k < 6; ++k) acc[j][i] += b[i * 6 + k] * xv[k];
-          }
-        }
-      }
-      #pragma unroll
-      for (int j = 0; j < 3; ++j) {
-        if (j0 + j < nv && !(skip && skip[j0 + j])) {
-          double d = 0;
-          #pragma unroll
-          for (int i = 0; i < 6; ++i) { double v = acc[j][i]; for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o); acc[j][i] = v; }
-          if (lane == 0) {
-            for (int i = 0; i < 6; ++i) { Y[(size_t)(j0 + j) * nc6 + 6 * a + i] = acc[j][i]; d += acc[j][i] * X[(size_t)(j0 + j) * nc6 + 6 * a + i]; }
-            if (dot_base >= 0) S.wpart[threadIdx.x >> 5][dot_base + j0 + j] += d;
-          }
-        }
-      }
-    }
-  }
-}
-
-__global__ void __launch_bounds__(PCG2_THREADS) pcg2_kernel(Pcg2Args A) {
-  cg::grid_group grid = cg::this_grid();
-  extern __shared__ unsigned char pcg2_smem_raw[];
-  Pcg2Smem &S = *reinterpret_cast<Pcg2Smem *>(pcg2_smem_raw);
-  const int tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
-  const size_t nc6 = 6 * (size_t)A.n_poses;
-  const int nw = A.nw;
-  if (threadIdx.x == 0) {
-    int n = 1; S.rhs_col[0] = -1;
-    for (int q = 0; q < A.ni8; ++q) if ((A.intr_mask[q / KI] >> (q % KI)) & 1) { if (n < MAXRHS) S.rhs_col[n++] = q; }
-    S.nrhs = n;
-  }
-  __syncthreads();
-  const int nrhs = S.nrhs;
-  // ---- coarse operator E = W' Scc W, explicit inverse (nw <= 7)
-  if (nw > 0) {
-    spmv_multi(A, S, A.W, A.AW, nw, nullptr, -1);
-    grid.sync();
-    vsum_begin(S, nw * nw);
-    for (int a = 0; a < nw; ++a) for (int b = 0; b < nw; ++b) {
-      double v = 0; for (size_t i = tid; i < nc6; i += nt) v += A.W[a * nc6 + i] * A.AW[b * nc6 + i];
-      warp_acc(S, v, a * nw + b);
-    }
-    vsum_end(grid, S, nw * nw, A.part);
-    if (threadIdx.x == 0) {                 // Gauss-Jordan inverse (symmetrised input), scratch in S.T
-      double (*M)[33] = S.T;
-      for (int a = 0; a < nw; ++a) for (int b = 0; b < nw; ++b) { M[a][b] = 0.5 * (S.tot[a * nw + b] + S.tot[b * nw + a]); M[a][nw + b] = a == b ? 1.0 : 0.0; }
-      for (int c = 0; c < nw; ++c) {
-        int piv = c; for (int r2 = c + 1; r2 < nw; ++r2) if (fabs(M[r2][c]) > fabs(M[piv][c])) piv = r2;
-        if (piv != c) for (int q = 0; q < 2 * nw; ++q) { const double t2 = M[c][q]; M[c][q] = M[piv][q]; M[piv][q] = t2; }
-        const double d = M[c][c];
-        for (int q = 0; q < 2 * nw; ++q) M[c][q] /= d;
-        for (int r2 = 0; r2 < nw; ++r2) if (r2 != c) { const double f = M[r2][c]; if (f != 0.0) for (int q = 0; q < 2 * nw; ++q) M[r2][q] -= f * M[c][q]; }
-      }
-      for (int a = 0; a < nw; ++a) for (int b = 0; b < nw; ++b) S.Einv[a * nw + b] = M[a][nw + b];
-    }
-    __syncthreads();
-  }
-  // ---- init: X = 0, R = B, |b|^2
-  vsum_begin(S, nrhs);
-  for (int j = 0; j < nrhs; ++j) {
-    const double *src = j == 0 ? A.rhs : A.Sci + (size_t)S.rhs_col[j] * nc6;
-    double v = 0;
-    for (size_t i = tid; i < nc6; i += nt) { const double b = src[i]; A.X[j * nc6 + i] = 0.0; A.Rv[j * nc6 + i] = b; v += b * b; }
-    warp_acc(S, v, j);
-  }
-  vsum_end(grid, S, nrhs, A.part);
-  if (threadIdx.x < nrhs) { const int j = threadIdx.x; S.bb[j] = S.tot[j]; S.done[j] = !(S.tot[j] > 0.0); S.alpha[j] = 0; S.beta[j] = 0; S.rz[j] = 0; }
-  if (threadIdx.x == 0) { S.worst = 0; S.all_done = 0; }
-  __syncthreads();
-  int it = 0;
-  for (;;) {
-    // (a) coarse components c_j = W' r_j
-    if (nw > 0) {
-      vsum_begin(S, nrhs * nw);
-      for (int j = 0; j < nrhs; ++j) {
-        if (S.done[j]) continue;
-        for (int a = 0; a < nw; ++a) { double v = 0; for (size_t i = tid; i < nc6; i += nt) v += A.W[a * nc6 + i] * A.Rv[j * nc6 + i]; warp_acc(S, v, j * nw + a); }
-      }
-      vsum_end(grid, S, nrhs * nw, A.part);
-    }
-    // (b) z = Minv r + W Einv c ;  r'z
-    vsum_begin(S, nrhs);
-    for (int j = 0; j < nrhs; ++j) {
-      if (S.done[j]) continue;
-      double coef[MAXW];
-      #pragma unroll
-      for (int a = 0; a < MAXW; ++a) { double c = 0; if (a < nw) for (int b = 0; b < nw; ++b) c += S.Einv[a * nw + b] * S.tot[j * nw + b]; coef[a] = c; }
-      double v = 0;
-      for (size_t i = tid; i < nc6; i += nt) {
-        const size_t a6 = i / 6; const int k = (int)(i % 6); const double *M = A.Minv_c + 36 * a6 + 6 * k; const double *rb = A.Rv + j * nc6 + 6 * a6;
-        double zz = M[0] * rb[0] + M[1] * rb[1] + M[2] * rb[2] + M[3] * rb[3] + M[4] * rb[4] + M[5] * rb[5];
-        #pragma unroll
-        for (int a = 0; a < MAXW; ++a) if (a < nw) zz += A.W[a * nc6 + i] * coef[a];
-        A.Zv[j * nc6 + i] = zz; v += zz * A.Rv[j * nc6 + i];
-      }
-      warp_acc(S, v, j);
-    }
-    vsum_end(grid, S, nrhs, A.part);
-    if (threadIdx.x < nrhs) { const int j = threadIdx.x; if (!S.done[j]) { const double rzn = S.tot[j]; S.beta[j] = it == 0 ? 0.0 : rzn / S.rz[j]; S.rz[j] = rzn; } }
-    __syncthreads();
-    // (c) p = z + beta p
-    for (int j = 0; j < nrhs; ++j) {
-      if (S.done[j]) continue;
-      if (it == 0) { for (size_t i = tid; i < nc6; i += nt) A.Pv[j * nc6 + i] = A.Zv[j * nc6 + i]; }
-      else { const double bt = S.beta[j]; for (size_t i = tid; i < nc6; i += nt) A.Pv[j * nc6 + i] = A.Zv[j * nc6 + i] + bt * A.Pv[j * nc6 + i]; }
-    }
-    grid.sync();
-    if (it >= A.max_iter) break;
-    // (d) w = Scc p ; p'w (accumulated inside the SpMV)
-    vsum_begin(S, nrhs);
-    spmv_multi(A, S, A.Pv, A.Wv, nrhs, S.done, 0);
-    vsum_end(grid, S, nrhs, A.part);            // its grid.sync also publishes Wv
-    if (threadIdx.x < nrhs) { const int j = threadIdx.x; S.alpha[j] = S.done[j] ? 0.0 : S.rz[j] / S.tot[j]; }
-    __syncthreads();
-    // (e) x += alpha p ; r -= alpha w ; |r|^2
-    vsum_begin(S, nrhs);
-    for (int j = 0; j < nrhs; ++j) {
-      if (S.done[j]) continue;
-      const double al = S.alpha[j]; double v = 0;
-      for (size_t i = tid; i < nc6; i += nt) { A.X[j * nc6 + i] += al * A.Pv[j * nc6 + i]; const double rn = A.Rv[j * nc6 + i] - al * A.Wv[j * nc6 + i]; A.Rv[j * nc6 + i] = rn; v += rn * rn; }
-      warp_acc(S, v, j);
-    }
-    vsum_end(grid, S, nrhs, A.part);
-    ++it;
-    if (threadIdx.x == 0) {
-      int ad = 1; double wmax = 0;
-      for (int j = 0; j < nrhs; ++j) if (!S.done[j]) { const double rel2 = S.tot[j] / S.bb[j]; wmax = fmax(wmax, rel2); if (!(rel2 > A.tol * A.tol)) S.done[j] = 1; else ad = 0; }
-      S.all_done = ad; S.worst = fmax(wmax, 0.0);
-    }
-    __syncthreads();
-    if (S.all_done) break;
-  }
-  // ---- border: (Sii - Sci Y2) zi = bi - Sci y1 ; zc = y1 - Y2 zi
-  const int k = nrhs - 1;
-  if (k > 0) {
-    for (int a = 0; a < k; ++a) {                     // one reduction round per row: k+1 <= 33 values
-      vsum_begin(S, k + 1);
-      const double *row = A.Sci + (size_t)S.rhs_col[1 + a] * nc6;
-      for (int b = 0; b <= k; ++b) {                  // b == k -> X[0]
-        const double *x = A.X + (size_t)(b == k ? 0 : 1 + b) * nc6;
-        double v = 0; for (size_t i = tid; i < nc6; i += nt) v += row[i] * x[i];
-        warp_acc(S, v, b);
-      }
-      vsum_end(grid, S, k + 1, A.part);
-      if (threadIdx.x <= k) {
-        const int b = threadIdx.x;
-        if (b < k) S.T[a][b] = A.Sii[(size_t)S.rhs_col[1 + a] * A.ni8 + S.rhs_col[1 + b]] - S.tot[b];
-        else S.T[a][k] = A.rhs[nc6 + S.rhs_col[1 + a]] - S.tot[k];
-      }
-      __syncthreads();
-    }
-    if (threadIdx.x == 0) {        // Gaussian elimination with partial pivoting (k <= 32), on the symmetrised T
-      for (int a = 0; a < k; ++a) for (int b = a + 1; b < k; ++b) { const double m = 0.5 * (S.T[a][b] + S.T[b][a]); S.T[a][b] = m; S.T[b][a] = m; }
-      for (int c = 0; c < k; ++c) {
-        int piv = c; for (int r2 = c + 1; r2 < k; ++r2) if (fabs(S.T[r2][c]) > fabs(S.T[piv][c])) piv = r2;
-        if (piv != c) for (int q = 0; q <= k; ++q) { const double t2 = S.T[c][q]; S.T[c][q] = S.T[piv][q]; S.T[piv][q] = t2; }
-        for (int r2 = c + 1; r2 < k; ++r2) { const double f = S.T[r2][c] / S.T[c][c]; for (int q = c; q <= k; ++q) S.T[r2][q] -= f * S.T[c][q]; }
-      }
-      for (int c = k - 1; c >= 0; --c) { double sacc = S.T[c][k]; for (int q = c + 1; q < k; ++q) sacc -= S.T[c][q] * S.zi[q]; S.zi[c] = sacc / S.T[c][c]; }
-    }
-    __syncthreads();
-  }
-  for (size_t i = tid; i < nc6; i += nt) { double v = A.X[i]; for (int a = 0; a < k; ++a) v -= A.X[(size_t)(1 + a) * nc6 + i] * S.zi[a]; A.z[i] = v; }
-  for (int q = tid; q < A.ni8; q += nt) { double v = 0; for (int a = 0; a < k; ++a) if (S.rhs_col[1 + a] == q) v = S.zi[a]; A.z[nc6 + q] = v; }
-  if (tid == 0) { A.out[0] = (double)it; A.out[1] = sqrt(S.worst); A.out[2] = sqrt(S.bb[0]); }
-}
-
 // ------------------------------------------------------------------------------ PCG v3 (aggregated coarse space)
-// Same block elimination of the intrinsics border as v2, but the coarse space of the two-level
+// Same block elimination of the intrinsics border as above, but the coarse space of the two-level
 // preconditioner is piecewise: the cameras are partitioned into aggregates (<= ~16 graph neighbours,
 // built on the host from the camera-pair structure) and every aggregate carries its own copy of the
 // <= 7 gauge generators.  Long camera chains drift by slowly varying similarity transforms — exactly
@@ -1773,170 +1462,15 @@ __global__ void coarse_assemble_kernel(const double *__restrict__ Scc, const int
   }
 }
 
-// Coarse operator setup in ONE cooperative kernel: blocked right-looking Cholesky of the symmetrised
-// E (+ tiny ridge) with a shared-memory tiled trailing update, T = (L^-1)' by one warp per column,
-// Einv = T T' (= L^-T L^-1) with the same tiled product.  E is <= ~1000^2, FP64 on the CUDA cores.
-constexpr int CNB = 32;          // panel width
-constexpr int CT = 64;           // output tile
-// C[i][j] (-)= sum_{k in [k0,k1)} A[i][k] B[j][k] for the CT x CT tile at (i0,j0); 256 threads, 4x4 outputs each
-// (rows i0 + ty + 16 q, cols j0 + tx + 16 q: conflict-free shared-memory reads).  sm: 2 * CT * (CNB+1) doubles.
-// MODE 0: C[i][j] -= acc (lower part), 1: C[i][j] = C[j][i] = acc (lower part, mirrored), 2: full tile to shared Cs[64][65]
-template <int MODE>
-__device__ __forceinline__ void tile_abt(double *__restrict__ C, const double *__restrict__ A, const double *__restrict__ B, int n,
-                                         int i0, int j0, int k0, int k1, double *sm) {
-  double (*As)[CNB + 1] = reinterpret_cast<double (*)[CNB + 1]>(sm);
-  double (*Bs)[CNB + 1] = reinterpret_cast<double (*)[CNB + 1]>(sm + CT * (CNB + 1));
-  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  double acc[4][4];
-  #pragma unroll
-  for (int p = 0; p < 4; ++p)
-    #pragma unroll
-    for (int q = 0; q < 4; ++q) acc[p][q] = 0.0;
-  for (int kp = k0; kp < k1; kp += CNB) {
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < CT * CNB; idx += 256) {
-      const int rr = idx / CNB, cc = idx % CNB, k = kp + cc;
-      As[rr][cc] = (i0 + rr < n && k < k1) ? A[(size_t)(i0 + rr) * n + k] : 0.0;
-      Bs[rr][cc] = (j0 + rr < n && k < k1) ? B[(size_t)(j0 + rr) * n + k] : 0.0;
-    }
-    __syncthreads();
-    #pragma unroll 8
-    for (int kk = 0; kk < CNB; ++kk) {
-      double av[4], bv[4];
-      #pragma unroll
-      for (int p = 0; p < 4; ++p) { av[p] = As[ty + 16 * p][kk]; bv[p] = Bs[tx + 16 * p][kk]; }
-      #pragma unroll
-      for (int p = 0; p < 4; ++p)
-        #pragma unroll
-        for (int q = 0; q < 4; ++q) acc[p][q] += av[p] * bv[q];
-    }
-  }
-  #pragma unroll
-  for (int p = 0; p < 4; ++p)
-    #pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      const int i = i0 + ty + 16 * p, j = j0 + tx + 16 * q;
-      if (MODE == 2) { C[(ty + 16 * p) * (CT + 1) + tx + 16 * q] = acc[p][q]; }
-      else if (i < n && j < n && j <= i) {
-        if (MODE == 0) C[(size_t)i * n + j] -= acc[p][q]; else { C[(size_t)i * n + j] = acc[p][q]; C[(size_t)j * n + i] = acc[p][q]; }
-      }
-    }
-}
-
-__global__ void __launch_bounds__(256) coarse_setup_kernel(double *__restrict__ E, int n, double *__restrict__ T, double *__restrict__ Einv, int *__restrict__ fail) {
-  cg::grid_group grid = cg::this_grid();
-  extern __shared__ double csm[];            // CNB*CNB + 2*CT*(CNB+1) + 2*CT*(CT+1) doubles
-  const int tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, gwarp = tid >> 5, nwarps = nt >> 5;
-  double *tsm = csm + CNB * CNB;
-  __shared__ double s_ridge;
-  for (long long idx = tid; idx < (long long)n * n; idx += nt) { const int i = (int)(idx / n), j = (int)(idx % n); if (j < i) E[(size_t)i * n + j] = 0.5 * (E[(size_t)i * n + j] + E[(size_t)j * n + i]); }
-  if (threadIdx.x == 0) { double mx = 0; for (int i = 0; i < n; ++i) mx = fmax(mx, E[(size_t)i * n + i]); s_ridge = 1e-15 * mx; }
-  grid.sync();
-  const double ridge = s_ridge;
-  for (int kb = 0; kb < n; kb += CNB) {
-    const int nb = min(CNB, n - kb);
-    // (1) every block factors the nb x nb diagonal block redundantly in shared memory
-    for (int idx = threadIdx.x; idx < nb * nb; idx += blockDim.x) { const int i = idx / nb, j = idx % nb; csm[i * CNB + j] = j <= i ? E[(size_t)(kb + i) * n + kb + j] + (i == j ? ridge : 0.0) : 0.0; }
-    __syncthreads();
-    if (wib == 0) {
-      for (int k = 0; k < nb; ++k) {
-        double d = csm[k * CNB + k];
-        if (!(d > 0.0) || !isfinite(d)) { if (lane == 0 && blockIdx.x == 0) atomicExch(fail, 4); d = 1.0; }
-        d = sqrt(d);
-        __syncwarp();
-        if (lane == 0) csm[k * CNB + k] = d;
-        for (int i = k + 1 + lane; i < nb; i += 32) csm[i * CNB + k] /= d;
-        __syncwarp();
-        for (int i = k + 1 + lane; i < nb; i += 32) { const double lik = csm[i * CNB + k]; for (int j = k + 1; j <= i; ++j) csm[i * CNB + j] -= lik * csm[j * CNB + k]; }
-        __syncwarp();
-      }
-    }
-    __syncthreads();
-    if (blockIdx.x == 0) for (int idx = threadIdx.x; idx < nb * nb; idx += blockDim.x) { const int i = idx / nb, j = idx % nb; if (j <= i) E[(size_t)(kb + i) * n + kb + j] = csm[i * CNB + j]; }
-    // (2) panel: L[i, kb:kb+nb] = A[i, kb:kb+nb] D^-T, one thread per row below the block
-    for (int i = kb + nb + tid; i < n; i += nt) {
-      double x[CNB];
-      #pragma unroll
-      for (int j = 0; j < CNB; ++j) x[j] = j < nb ? E[(size_t)i * n + kb + j] : 0.0;
-      #pragma unroll
-      for (int j = 0; j < CNB; ++j) if (j < nb) {
-        double v = x[j];
-        #pragma unroll
-        for (int q = 0; q < CNB; ++q) if (q < j) v -= x[q] * csm[j * CNB + q];
-        x[j] = v / csm[j * CNB + j];
-      }
-      #pragma unroll
-      for (int j = 0; j < CNB; ++j) if (j < nb) E[(size_t)i * n + kb + j] = x[j];
-    }
-    grid.sync();
-    // (3) trailing update, lower-triangular CT x CT tiles:  A22 -= L21 L21'
-    const int r0 = kb + nb, mt = (n - r0 + CT - 1) / CT;
-    for (int t = blockIdx.x; t < mt * mt; t += gridDim.x) {
-      const int bi = t / mt, bj = t % mt;
-      if (bj > bi) continue;
-      tile_abt<0>(E, E, E, n, r0 + bi * CT, r0 + bj * CT, kb, kb + nb, tsm);
-    }
-    grid.sync();
-  }
-  // T = (L^-1)' by blocks of CT: (a) invert the diagonal blocks in shared memory, (b) block column j of L^-1
-  // by forward substitution over block rows, one CTA per block column (tiled products), T stored transposed.
-  const int nbk = (n + CT - 1) / CT;
-  double *Ls = tsm + 2 * CT * (CNB + 1);                 // [CT][CT+1] scratch: a diagonal block of L, then S
-  double *Ds = Ls + CT * (CT + 1);                        // [CT][CT+1] inverse of a diagonal block
-  for (long long idx = tid; idx < (long long)n * n; idx += nt) T[idx] = 0.0;
-  grid.sync();
-  for (int bq = blockIdx.x; bq < nbk; bq += gridDim.x) {
-    const int o = bq * CT, m = min(CT, n - o);
-    for (int idx = threadIdx.x; idx < CT * CT; idx += blockDim.x) { const int r = idx / CT, cc = idx % CT; Ls[r * (CT + 1) + cc] = (r < m && cc <= r) ? E[(size_t)(o + r) * n + o + cc] : (r == cc ? 1.0 : 0.0); }
-    __syncthreads();
-    if (threadIdx.x < CT) {                                // column c of inv(L_bb): x_i = (delta - sum_{k<i} L_ik x_k) / L_ii
-      const int c = threadIdx.x;
-      for (int i = 0; i < CT; ++i) {
-        double v = i == c ? 1.0 : 0.0;
-        for (int k = c; k < i; ++k) v -= Ls[i * (CT + 1) + k] * Ds[k * (CT + 1) + c];
-        Ds[i * (CT + 1) + c] = i < c ? 0.0 : v / Ls[i * (CT + 1) + i];
-      }
-    }
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < CT * CT; idx += blockDim.x) { const int r = idx / CT, cc = idx % CT; if (r < m && cc < m && cc <= r) T[(size_t)(o + cc) * n + o + r] = Ds[r * (CT + 1) + cc]; }
-    __syncthreads();
-  }
-  grid.sync();
-  for (int bj = blockIdx.x; bj < nbk; bj += gridDim.x) {
-    for (int bi = bj + 1; bi < nbk; ++bi) {
-      // S = sum_{k in [bj*CT, bi*CT)} L[bi rows][k] * Linv[k][bj cols]  ==  tile of  L . T'   (T holds Linv transposed)
-      tile_abt<2>(Ls, E, T, n, bi * CT, bj * CT, bj * CT, bi * CT, tsm);
-      __syncthreads();
-      // Linv_ij = -inv(L_ii) S ; inv(L_ii) is in T (transposed): Dinv[r][q] = T[o_i + q][o_i + r]
-      const int oi = bi * CT, oj = bj * CT, mi = min(CT, n - oi), mj = min(CT, n - oj);
-      for (int idx = threadIdx.x; idx < CT * CT; idx += blockDim.x) { const int r = idx / CT, q = idx % CT; Ds[r * (CT + 1) + q] = (r < mi && q <= r) ? T[(size_t)(oi + q) * n + oi + r] : 0.0; }
-      __syncthreads();
-      for (int idx = threadIdx.x; idx < CT * CT; idx += blockDim.x) {
-        const int r = idx / CT, cc = idx % CT;
-        if (r < mi && cc < mj) { double v = 0; for (int q = 0; q <= r; ++q) v += Ds[r * (CT + 1) + q] * Ls[q * (CT + 1) + cc]; T[(size_t)(oj + cc) * n + oi + r] = -v; }
-      }
-      __syncthreads();
-      __threadfence();                                      // later block rows of this column read T written above
-    }
-  }
-  grid.sync();
-  // Einv = T T'  (T[i][k] = 0 for k < i, so the sum starts at the tile's first row index)
-  { const int mt = (n + CT - 1) / CT;
-    for (int t = blockIdx.x; t < mt * mt; t += gridDim.x) {
-      const int bi = t / mt, bj = t % mt;
-      if (bj > bi) continue;
-      tile_abt<1>(Einv, T, T, n, bi * CT, bj * CT, (bi * CT / CNB) * CNB, n, tsm);
-    } }
-}
-
-// Coarse operator inverse by blocked Gauss-Jordan, in place, ONE cooperative kernel (default).  The Cholesky route above
-// serialises on its triangular inverse (one CTA per block column); Gauss-Jordan does twice the flops but every
-// pivot step is a rank-32 update of the WHOLE matrix — 196 independent 64x64 tiles — between two grid syncs:
+// Coarse operator inverse by blocked Gauss-Jordan, in place, ONE cooperative kernel.  A blocked Cholesky with an
+// explicit triangular inverse serialises on that inverse (one CTA per block column; 2.46 vs 1.0 ms, DESIGN.md §4.3);
+// Gauss-Jordan does twice the flops but every pivot step is a rank-32 update of the WHOLE matrix — 196 independent
+// 64x64 tiles — between two grid syncs:
 //   phase 1 (every CTA): B = inv(A_KK) redundantly in shared memory; slices of  Cold = A[:,K] (copy),
 //                        H = B A[K,:],  Gn = -A[:,K] B  into scratch
 //   phase 2 (tiles):     A_ij <- A_ij - Cold_i H_j  (i,j not in K);  A_Kj <- H_j;  A_iK <- Gn_i;  A_KK <- B
 // A is symmetrised (+ tiny ridge) first; SPD input needs no pivoting (every pivot block is a Schur complement).
+constexpr int CT = 64;           // output tile
 constexpr int GJ_B = 32;
 __device__ __forceinline__ unsigned long long gtimer2() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
 #define GJ_LAP(k) do { if (tim && tid == 0) { const unsigned long long now_ = gtimer2(); tim[k] += now_ - tlast; tlast = now_; } } while (0)
@@ -2352,258 +1886,6 @@ __global__ void __launch_bounds__(PCG2_THREADS) pcg3_kernel(Pcg3Args P) {
   if (tid == 0) { A.out[0] = (double)it; A.out[1] = sqrt(S.worst); A.out[2] = sqrt(S.bb[0]); }
 }
 
-// ------------------------------------------------------------------------------ PCG v4 (aggregate-owned, 2 grid syncs per iteration)
-// Same mathematics as v3 (block elimination of the intrinsics border, M^-1 = blockdiag^-1 + Wa (Wa' Scc Wa)^-1 Wa'),
-// different ownership: CTA g owns aggregate g — its camera rows of the SpMV, its slices of every vector, its nw rows of
-// the coarse solve.  That removes two of the four grid-wide steps of an iteration:
-//   * the coarse solve needs no step of its own: every CTA stages the (tiny) coarse residual and computes only the
-//     nw rows y_g = Einv[g rows, :] c it needs itself (one L2 round trip: the row loads are all in flight together);
-//   * the coarse residual of the NEW r needs no step either: c_new = c - alpha Wa' w, and Wa' w of an aggregate is
-//     formed inside its CTA during the SpMV and published with the same grid sync that publishes p'w.
-// Per iteration:  [A] alpha; x += alpha p, r -= alpha w, |r|^2; c_new; y_g; z = Minv r + Wa y; r'z      -> sync
-//                 [B] beta, convergence test; w = Scc (z + beta p) on the fly, p'w, Wa' w of the aggregate -> sync
-// (v3: coarse solve -> sync, z -> sync, SpMV -> sync, update -> sync.)  Reductions are fixed-order.
-constexpr int PCG4_MAXCAM = 32;        // cameras per aggregate handled in place (aggregation keeps them <= ~16)
-__global__ void __launch_bounds__(PCG2_THREADS) pcg4_kernel(Pcg3Args P, double *__restrict__ Cv2, double *__restrict__ AW) {
-  cg::grid_group grid = cg::this_grid();
-  extern __shared__ unsigned char pcg2_smem_raw[];
-  Pcg2Smem &S = *reinterpret_cast<Pcg2Smem *>(pcg2_smem_raw);
-  double *sCv = reinterpret_cast<double *>(pcg2_smem_raw + sizeof(Pcg2Smem));     // [4][PCG3_NCO_MAX] coarse residual chunk
-  __shared__ double s_y[MAXW][MAXRHS];                                            // y_g of the aggregate being processed
-  __shared__ double s_aw[PCG2_THREADS / 32][4][MAXW];                             // per-warp Wa' w partials (one chunk of 4 rhs)
-  const Pcg2Args &A = P.base; const Coarse &C = P.C;
-  const int tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  constexpr int NWARP = PCG2_THREADS / 32;
-  const size_t nc6 = 6 * (size_t)A.n_poses;
-  const int nw = C.nw, nco = C.nco;
-  if (threadIdx.x == 0) {
-    int n = 1; S.rhs_col[0] = -1;
-    for (int q = 0; q < A.ni8; ++q) if ((A.intr_mask[q / KI] >> (q % KI)) & 1) { if (n < MAXRHS) S.rhs_col[n++] = q; }
-    S.nrhs = n;
-  }
-  __syncthreads();
-  const int nrhs = S.nrhs;
-  double *Pcur = A.Pv, *Pnext = P.Pv2;
-  double *Ccur = P.Cv, *Cnext = Cv2;               // coarse residual, ping-pong: [nrhs][nco]
-  // ---- init (own aggregates): X = 0, P = 0, W = 0, R = B, |b|^2, c = Wa' b, AW = 0
-  vsum_begin(S, nrhs);
-  for (int g = blockIdx.x; g < C.ng; g += gridDim.x) {
-    const int c0 = C.agg_start[g], ne = 6 * (C.agg_start[g + 1] - c0);
-    for (int j = wib; j < nrhs; j += NWARP) {
-      const double *src = j == 0 ? A.rhs : A.Sci + (size_t)S.rhs_col[j] * nc6;
-      double v = 0, cm[MAXW];
-      #pragma unroll
-      for (int m = 0; m < MAXW; ++m) cm[m] = 0.0;
-      for (int idx = lane; idx < ne; idx += 32) {
-        const size_t e = 6 * (size_t)C.agg_cams[c0 + idx / 6] + idx % 6; const double b = src[e];
-        A.X[j * nc6 + e] = 0.0; Pcur[j * nc6 + e] = 0.0; A.Wv[j * nc6 + e] = 0.0; A.Rv[j * nc6 + e] = b; v += b * b;
-        #pragma unroll
-        for (int m = 0; m < MAXW; ++m) if (m < nw) cm[m] += A.W[m * nc6 + e] * b;
-      }
-      warp_acc(S, v, j);
-      #pragma unroll
-      for (int m = 0; m < MAXW; ++m) if (m < nw) {
-        double cv = cm[m]; for (int o = 16; o > 0; o >>= 1) cv += __shfl_xor_sync(0xffffffffu, cv, o);
-        if (lane == 0) { Ccur[(size_t)j * nco + g * nw + m] = cv; AW[(size_t)j * nco + g * nw + m] = 0.0; }
-      }
-    }
-  }
-  vsum_end(grid, S, nrhs, A.part);
-  if (threadIdx.x < nrhs) { const int j = threadIdx.x; S.bb[j] = S.tot[j]; S.done[j] = !(S.tot[j] > 0.0); S.alpha[j] = 0; S.beta[j] = 0; S.rz[j] = 0; }
-  if (threadIdx.x == 0) { S.worst = 0; S.all_done = 0; }
-  __syncthreads();
-  int it = 0;
-  unsigned long long tlast = P.tim ? gtimer() : 0ull;
-  for (;;) {
-    // ================================================================= [A]
-    vsum_begin(S, 2 * nrhs);
-    for (int j0 = 0; j0 < nrhs; j0 += 4) {
-      const int nj = min(4, nrhs - j0);
-      // coarse residual of the new r for ALL aggregates: c_new = c - alpha Wa'w  (every CTA forms the whole (tiny) vector;
-      // the owner of an aggregate also stores its entries for the next iteration)
-      if (nco > 0) {
-        __syncthreads();
-        for (int k = threadIdx.x; k < nco; k += PCG2_THREADS) {
-          const int g = k / nw; const bool mine = (g % (int)gridDim.x) == (int)blockIdx.x;
-          #pragma unroll
-          for (int j = 0; j < 4; ++j) if (j < nj) {
-            const size_t o = (size_t)(j0 + j) * nco + k;
-            const double cn = __ldcg(Ccur + o) - S.alpha[j0 + j] * __ldcg(AW + o);
-            sCv[j * PCG3_NCO_MAX + k] = cn;
-            if (mine) Cnext[o] = cn;
-          }
-        }
-        __syncthreads();
-      }
-      PCG_LAP(0);
-      for (int g = blockIdx.x; g < C.ng; g += gridDim.x) {
-        const int c0 = C.agg_start[g], ne = 6 * (C.agg_start[g + 1] - c0);
-        // y_g[m][j] = Einv[g nw + m, :] . c_new[j, :]   (warp m)
-        if (nco > 0) {
-          for (int m = wib; m < nw; m += NWARP) {
-            const double *er = P.Einv + (size_t)(g * nw + m) * nco;
-            double ev[PCG3_NCO_MAX / 32];
-            #pragma unroll
-            for (int q = 0; q < PCG3_NCO_MAX / 32; ++q) { const int k = lane + 32 * q; ev[q] = k < nco ? __ldcg(er + k) : 0.0; }
-            double acc[4] = {0, 0, 0, 0};
-            #pragma unroll
-            for (int q = 0; q < PCG3_NCO_MAX / 32; ++q) { const int k = lane + 32 * q;
-              if (k < nco) {
-                #pragma unroll
-                for (int j = 0; j < 4; ++j) if (j < nj) acc[j] += ev[q] * sCv[j * PCG3_NCO_MAX + k]; } }
-            #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              double v = acc[j]; for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-              if (lane == 0 && j < nj) s_y[m][j0 + j] = v;
-            }
-          }
-          __syncthreads();
-          PCG_LAP(1);
-        }
-        // own slices: x += alpha p ; r -= alpha w ; |r|^2 ; z = Minv r + Wa y ; r'z       (warp per right-hand side)
-        for (int j = j0 + wib; j < j0 + nj; j += NWARP) {
-          if (S.done[j]) continue;
-          const double al = S.alpha[j];
-          double y[MAXW];
-          #pragma unroll
-          for (int m = 0; m < MAXW; ++m) y[m] = (m < nw && nco > 0) ? s_y[m][j] : 0.0;
-          double rr = 0, rz = 0;
-          // (r of a camera is needed whole for Minv r: update it first, then form z)
-          for (int idx = lane; idx < ne; idx += 32) {
-            const size_t e = 6 * (size_t)C.agg_cams[c0 + idx / 6] + idx % 6;
-            A.X[j * nc6 + e] += al * Pcur[j * nc6 + e];
-            const double rn = A.Rv[j * nc6 + e] - al * A.Wv[j * nc6 + e]; A.Rv[j * nc6 + e] = rn; rr += rn * rn;
-          }
-          __syncwarp();
-          for (int idx = lane; idx < ne; idx += 32) {
-            const size_t cam = C.agg_cams[c0 + idx / 6]; const int k = idx % 6; const size_t e = 6 * cam + k;
-            const double *rb = A.Rv + j * nc6 + 6 * cam;
-            const double2 *M2 = reinterpret_cast<const double2 *>(A.Minv_c + 36 * cam + 6 * k), *r2 = reinterpret_cast<const double2 *>(rb);
-            const double2 m0 = M2[0], m1 = M2[1], m2 = M2[2], b0 = r2[0], b1 = r2[1], b2 = r2[2];
-            double zz = m0.x * b0.x + m0.y * b0.y + m1.x * b1.x + m1.y * b1.y + m2.x * b2.x + m2.y * b2.y;
-            #pragma unroll
-            for (int m = 0; m < MAXW; ++m) if (m < nw) zz += A.W[m * nc6 + e] * y[m];
-            A.Zv[j * nc6 + e] = zz; rz += zz * rb[k];
-          }
-          warp_acc(S, rz, j); warp_acc(S, rr, nrhs + j);
-        }
-        __syncthreads();                                   // s_y is reused by the next aggregate / chunk
-      }
-    }
-    PCG_LAP(2);
-    vsum_end(grid, S, 2 * nrhs, A.part);
-    PCG_LAP(3);
-    { double *t2 = Ccur; Ccur = Cnext; Cnext = t2; }
-    if (threadIdx.x < nrhs) { const int j = threadIdx.x; if (!S.done[j]) { const double rzn = S.tot[j]; S.beta[j] = it == 0 ? 0.0 : rzn / S.rz[j]; S.rz[j] = rzn; } }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      int ad = 1; double wmax = 0;
-      for (int j = 0; j < nrhs; ++j) if (!S.done[j]) { const double rel2 = S.tot[nrhs + j] / S.bb[j]; wmax = fmax(wmax, rel2); if (!(rel2 > A.tol * A.tol)) S.done[j] = 1; else ad = 0; }
-      S.all_done = ad; if (it > 0) S.worst = wmax;
-    }
-    __syncthreads();
-    if (S.all_done || it >= A.max_iter) break;
-    // ================================================================= [B]  w = Scc (z + beta p) ; p'w ; Wa' w
-    vsum_begin(S, nrhs);
-    for (int j0 = 0; j0 < nrhs; j0 += 4) {
-      const int nj = min(4, nrhs - j0);
-      for (int g = blockIdx.x; g < C.ng; g += gridDim.x) {
-        const int c0 = C.agg_start[g], ncam = C.agg_start[g + 1] - c0;
-        for (int i = threadIdx.x; i < NWARP * 4 * MAXW; i += PCG2_THREADS) (&s_aw[0][0][0])[i] = 0.0;
-        __syncthreads();
-        for (int ci = wib; ci < ncam; ci += NWARP) {
-          const int a = C.agg_cams[c0 + ci];
-          double acc[4][6];
-          #pragma unroll
-          for (int j = 0; j < 4; ++j)
-            #pragma unroll
-            for (int i = 0; i < 6; ++i) acc[j][i] = 0.0;
-          for (int e = A.rowptr[a] + lane; e < A.rowptr[a + 1]; e += 32) {
-            const double *blk = A.Scc + 36 * (size_t)e; const int cb = 6 * A.cols[e];
-            double b[36];
-            #pragma unroll
-            for (int i = 0; i < 9; ++i) ldg256(blk + 4 * i, b[4 * i], b[4 * i + 1], b[4 * i + 2], b[4 * i + 3]);
-            #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              if (j < nj && !S.done[j0 + j]) {
-                const size_t off = (size_t)(j0 + j) * nc6 + cb; const double bt = S.beta[j0 + j];
-                const double2 *zp = reinterpret_cast<const double2 *>(A.Zv + off), *pp = reinterpret_cast<const double2 *>(Pcur + off);
-                const double2 z0 = zp[0], z1 = zp[1], z2 = zp[2], q0 = pp[0], q1 = pp[1], q2 = pp[2];
-                const double xv[6] = {z0.x + bt * q0.x, z0.y + bt * q0.y, z1.x + bt * q1.x, z1.y + bt * q1.y, z2.x + bt * q2.x, z2.y + bt * q2.y};
-                #pragma unroll
-                for (int i = 0; i < 6; ++i)
-                  #pragma unroll
-                  for (int k = 0; k < 6; ++k) acc[j][i] += b[i * 6 + k] * xv[k];
-              }
-            }
-          }
-          #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            if (j < nj && !S.done[j0 + j]) {
-              #pragma unroll
-              for (int i = 0; i < 6; ++i) { double v = acc[j][i]; for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o); acc[j][i] = v; }
-              if (lane == 0) {
-                const size_t off = (size_t)(j0 + j) * nc6 + 6 * (size_t)a; const double bt = S.beta[j0 + j];
-                double d = 0;
-                for (int i = 0; i < 6; ++i) { const double pv = A.Zv[off + i] + bt * Pcur[off + i]; Pnext[off + i] = pv; A.Wv[off + i] = acc[j][i]; d += acc[j][i] * pv; }
-                S.wpart[wib][j0 + j] += d;
-                for (int m = 0; m < nw; ++m) { double t = 0; for (int i = 0; i < 6; ++i) t += A.W[m * nc6 + 6 * (size_t)a + i] * acc[j][i]; s_aw[wib][j][m] += t; }
-              }
-            }
-          }
-        }
-        __syncthreads();
-        for (int i = threadIdx.x; i < nj * nw; i += PCG2_THREADS) {
-          const int j = i / nw, m = i % nw;
-          if (!S.done[j0 + j]) { double t = 0; for (int w = 0; w < NWARP; ++w) t += s_aw[w][j][m]; AW[(size_t)(j0 + j) * nco + g * nw + m] = t; }
-        }
-        __syncthreads();
-      }
-    }
-    PCG_LAP(4);
-    vsum_end(grid, S, nrhs, A.part);              // its grid.sync also publishes Wv, Pnext and AW
-    PCG_LAP(5);
-    { double *t2 = Pcur; Pcur = Pnext; Pnext = t2; }
-    if (threadIdx.x < nrhs) { const int j = threadIdx.x; S.alpha[j] = S.done[j] ? 0.0 : S.rz[j] / S.tot[j]; }
-    __syncthreads();
-    ++it;
-  }
-  // ---- border: (Sii - Sci Y2) zi = bi - Sci y1 ; zc = y1 - Y2 zi      (as v3)
-  const int k = nrhs - 1;
-  if (k > 0) {
-    for (int a = 0; a < k; ++a) {
-      vsum_begin(S, k + 1);
-      const double *row = A.Sci + (size_t)S.rhs_col[1 + a] * nc6;
-      for (int b = 0; b <= k; ++b) {
-        const double *x = A.X + (size_t)(b == k ? 0 : 1 + b) * nc6;
-        double v = 0; for (size_t i = tid; i < nc6; i += nt) v += row[i] * x[i];
-        warp_acc(S, v, b);
-      }
-      vsum_end(grid, S, k + 1, A.part);
-      if (threadIdx.x <= k) {
-        const int b = threadIdx.x;
-        if (b < k) S.T[a][b] = A.Sii[(size_t)S.rhs_col[1 + a] * A.ni8 + S.rhs_col[1 + b]] - S.tot[b];
-        else S.T[a][k] = A.rhs[nc6 + S.rhs_col[1 + a]] - S.tot[k];
-      }
-      __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-      for (int a = 0; a < k; ++a) for (int b = a + 1; b < k; ++b) { const double m = 0.5 * (S.T[a][b] + S.T[b][a]); S.T[a][b] = m; S.T[b][a] = m; }
-      for (int c = 0; c < k; ++c) {
-        int piv = c; for (int r2 = c + 1; r2 < k; ++r2) if (fabs(S.T[r2][c]) > fabs(S.T[piv][c])) piv = r2;
-        if (piv != c) for (int q = 0; q <= k; ++q) { const double t2 = S.T[c][q]; S.T[c][q] = S.T[piv][q]; S.T[piv][q] = t2; }
-        for (int r2 = c + 1; r2 < k; ++r2) { const double f = S.T[r2][c] / S.T[c][c]; for (int q = c; q <= k; ++q) S.T[r2][q] -= f * S.T[c][q]; }
-      }
-      for (int c = k - 1; c >= 0; --c) { double sacc = S.T[c][k]; for (int q = c + 1; q < k; ++q) sacc -= S.T[c][q] * S.zi[q]; S.zi[c] = sacc / S.T[c][c]; }
-    }
-    __syncthreads();
-  }
-  for (size_t i = tid; i < nc6; i += nt) { double v = A.X[i]; for (int a = 0; a < k; ++a) v -= A.X[(size_t)(1 + a) * nc6 + i] * S.zi[a]; A.z[i] = v; }
-  for (int q = tid; q < A.ni8; q += nt) { double v = 0; for (int a = 0; a < k; ++a) if (S.rhs_col[1 + a] == q) v = S.zi[a]; A.z[nc6 + q] = v; }
-  if (tid == 0) { A.out[0] = (double)it; A.out[1] = sqrt(S.worst); A.out[2] = sqrt(S.bb[0]); }
-}
-
 // ------------------------------------------------------------------------------ PCG v5 (shared-memory resident)
 // The v3 iteration is four grid-wide phases of three or four DEPENDENT L2 round trips each (every vector element a
 // CTA touches was last written by another SM): ~26 us per iteration at 1000 cameras for ~0.3 us of arithmetic.
@@ -2614,7 +1896,8 @@ __global__ void __launch_bounds__(PCG2_THREADS) pcg4_kernel(Pcg3Args P, double *
 //   [B] read  beta-partials + z, p of the neighbour cameras (one trip) write  p of its cameras, p'w partials, Wa'w
 // i.e. two grid barriers and two L2 round trips; the coarse solve (its nw rows of Einv, fetched into registers in the
 // shadow of the Wa'w read), the block-Jacobi step, the vector updates and the SpMV arithmetic are local.
-// Same recurrences as v4 (c_new = c - alpha Wa'w), same stopping rule and iteration count as v3.
+// The coarse residual of the new r is not recomputed but updated, c_new = c - alpha Wa'w, with Wa'w formed during the
+// SpMV and published by the same barrier as p'w.  Same stopping rule and iteration count as v3.
 constexpr int PCG5_NR = 4;            // right-hand sides held in shared memory (1 + free intrinsic columns)
 constexpr int PCG5_MC = 21;           // cameras per aggregate (aggregation keeps them <= ~16; 2000-camera scenes reach 17-20)
 constexpr int PCG5_ST = ((PCG5_MC * 6 + 31) / 32) * 32;   // per-rhs thread stride: a warp never straddles two right-hand sides

@@ -41,7 +41,6 @@ constexpr int B_STAGE_BYTES = B_BYTES + CK_BYTES;
 constexpr int SMEM_BYTES = A_STAGES * A_BYTES + B_STAGES * B_STAGE_BYTES + 1024 /*align slack*/ + 2048 /*merge*/ + 256 /*barriers*/;
 constexpr int TC_THREADS = 320;  // warp0 TMA, warp1 MMA, warps 2-5 / 6-9 epilogue for even / odd tiles
 constexpr int KEY_MIN = INT_MIN;
-constexpr int MATCH_NSPLIT_DEFAULT = 2;
 
 struct Unit { uint32_t q_row, db_row, n_db_tiles, out_off; };   // one (pair, 128-query tile); n_db_tiles = tiles | (rows per group / 32) << 20
 constexpr uint32_t UNIT_TILES_MASK = 0xFFFFFu;
@@ -101,7 +100,6 @@ __device__ __forceinline__ void chunk_update(const int32_t (&r)[32], uint32_t ck
   k1 = max(k1, gm);
 }
 
-template <int DRAIN_ONLY>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 match_tc_kernel(const __grid_constant__ CUtensorMap tmap, const int32_t *__restrict__ ckey,
                 const Unit *__restrict__ units, uint32_t n_units, int2 *__restrict__ k12) {
@@ -201,10 +199,10 @@ match_tc_kernel(const __grid_constant__ CUtensorMap tmap, const int32_t *__restr
         for (int c = 0; c < TILE_DB / 32; c += 2) {
           tmem_ld_wait_dep(ra);
           tmem_ld_32x32(taddr + (c + 1) * 32, rb);
-          if (!DRAIN_ONLY) chunk_update(ra, ck + c * 128, k1, k2);
+          chunk_update(ra, ck + c * 128, k1, k2);
           tmem_ld_wait_dep(rb);
           if (c + 2 < TILE_DB / 32) tmem_ld_32x32(taddr + (c + 2) * 32, ra);
-          if (!DRAIN_ONLY) chunk_update(rb, ck + (c + 1) * 128, k1, k2);
+          chunk_update(rb, ck + (c + 1) * 128, k1, k2);
         }
         tc_fence_before();
         __syncwarp();
@@ -230,10 +228,10 @@ match_tc_kernel(const __grid_constant__ CUtensorMap tmap, const int32_t *__restr
 
 
 // --------------------------------------------------------------------------------- tcgen05 kernel, fifth K-slice
-// The shipped kernel.  match_tc_kernel above spends 1 IMAD per accumulator on key = 512*dot + ckey[column]; here the
-// per-column constant rides in the MMA instead: a fifth K=32 slice multiplies a CONSTANT A tile (weights
-// 1, 255 x 15, 1, 255 x 15 in every row) with 32 signed "digits" per database row (u8 x s8, its own instruction
-// descriptor) so that the accumulator is   acc = q.b - h(b) + c0(image),  h = ceil(|b|^2 / 2).
+// The shipped kernel (match_dig2_kernel below).  match_tc_kernel above spends 1 IMAD per accumulator on
+// key = 512*dot + ckey[column]; here the per-column constant rides in the MMA instead: a fifth K=32 slice multiplies a
+// CONSTANT A tile (weights 1, 255 x 15, 1, 255 x 15 in every row) with 32 signed "digits" per database row (u8 x s8,
+// its own instruction descriptor) so that the accumulator is   acc = q.b - h(b) + c0(image),  h = ceil(|b|^2 / 2).
 // The epilogue is then a pure running max (VIMNMX3: half an instruction per accumulator) and ONE key per 32-column
 // chunk, key = 256 * max + group.  What is lost is the parity of |b|^2:  2 q.b - |b|^2 = 2 acc - 2 c0 + p, p in
 // {0, 1}; the finalize kernel works with the two-sided bound and falls back to an exact scan of the whole database
@@ -241,7 +239,7 @@ match_tc_kernel(const __grid_constant__ CUtensorMap tmap, const int32_t *__restr
 // most negative digit vector (DIG_PAD), strictly below every real column, and zero descriptors.
 // Digit range: v = c0 - h must lie in [DIG_VMIN, DIG_VMAX]; omvg_match_prepare picks c0 per image and uses this
 // kernel only if every image fits (|b|^2 spread <= 3.9 M inside an image: always true for SIFT, whose |b|^2 is
-// ~2.6e5); otherwise match_tc_kernel runs.  NSPLIT = epilogue warps per TMEM lane quarter and accumulator.
+// ~2.6e5); otherwise match_tc_kernel runs.
 constexpr int DIG_LEN = 32;
 constexpr int DG_BYTES = TILE_DB * DIG_LEN;                      //  8 KB of digits per database tile
 constexpr int B5_STAGE_BYTES = B_BYTES + DG_BYTES;               // 40 KB
@@ -249,9 +247,6 @@ constexpr int ACONST_BYTES = TILE_Q * DIG_LEN;                   //  4 KB
 constexpr int DIG_PAD = -128 * 2 - 128 * 255 * 30;               // -979456: all 32 digits = -128
 constexpr int DIG_VMIN = -979328, DIG_VMAX = 971676;             // v = d0 + 255 M, d0 in [-128, 126], M in [-3840, 3810]
 constexpr int DIG_SPREAD_MAX = DIG_VMAX - DIG_VMIN;              // 1 951 004 (in units of h)
-template <int NSPLIT> constexpr int smem5_bytes() {
-  return A_STAGES * A_BYTES + B_STAGES * B5_STAGE_BYTES + ACONST_BYTES + 1024 /*align slack*/ + 2 * (2 * NSPLIT - 1) * TILE_Q * 8 /*merge*/ + 256 /*barriers*/;
-}
 
 // per-image min / max of h = ceil(|row|^2 / 2) over the real rows (one block per image)
 __global__ void prep_minmax_kernel(const int32_t *__restrict__ norm, const uint32_t *__restrict__ img_row0,
@@ -322,168 +317,21 @@ __device__ __forceinline__ uint64_t make_kmajor_sw32_desc(uint32_t smem_addr) {
   return d;
 }
 
-template <int NSPLIT, bool DRAIN_ONLY>
-__global__ void __launch_bounds__(64 + 256 * NSPLIT, 1)
-match_dig_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_dig,
-                 const Unit *__restrict__ units, uint32_t n_units, int2 *__restrict__ k12) {
-  constexpr int NMERGE = 2 * NSPLIT - 1;               // partial top-2 lists merged by the first warps of a row
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t *a_smem = smem;                                        // [A_STAGES][16 KB]
-  uint8_t *b_smem = smem + A_STAGES * A_BYTES;                   // [B_STAGES][32 KB descriptors + 8 KB digits]
-  uint8_t *aconst = b_smem + B_STAGES * B5_STAGE_BYTES;          // [128][32 B] constant weights
-  int2 *merge = reinterpret_cast<int2 *>(aconst + ACONST_BYTES); // [2][NMERGE][128]
-  uint64_t *bars = reinterpret_cast<uint64_t *>(merge + 2 * NMERGE * TILE_Q);
-  uint64_t *full_a = bars, *empty_a = bars + 2, *full_b = bars + 4, *empty_b = bars + 8;
-  uint64_t *tmem_full = bars + 12, *tmem_empty = bars + 14;
-  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 16);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap); prefetch_tmap(&tmap_dig);
-    for (int i = 0; i < A_STAGES; ++i) { mbar_init(&full_a[i], 1); mbar_init(&empty_a[i], 1); }
-    for (int i = 0; i < B_STAGES; ++i) { mbar_init(&full_b[i], 1); mbar_init(&empty_b[i], 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 4 * NSPLIT); }
-    fence_barrier_init();
-  }
-  // weights of the fifth slice: both 16-byte halves of every row are {1, 255 x 15}, so the swizzle cannot matter
-  for (int i = threadIdx.x; i < ACONST_BYTES / 16; i += blockDim.x)
-    reinterpret_cast<uint4 *>(aconst)[i] = make_uint4(0xFFFFFF01u, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
-  fence_proxy_async();
-  if (warp == 2) tmem_alloc(tmem_slot, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ===================================================================== TMA producer
-    if (lane == 0) {
-      uint32_t g = 0, ul = 0;
-      for (uint32_t u = blockIdx.x; u < n_units; u += gridDim.x, ++ul) {
-        const Unit un = units[u];
-        const uint32_t as = ul & 1, n_tiles = un.n_db_tiles & UNIT_TILES_MASK;
-        mbar_wait(&empty_a[as], ((ul >> 1) & 1) ^ 1);
-        mbar_arrive_expect_tx(&full_a[as], A_BYTES);
-        tma_load_2d(a_smem + as * A_BYTES, &tmap, 0, (int)un.q_row, &full_a[as]);
-        for (uint32_t t = 0; t < n_tiles; ++t, ++g) {
-          const uint32_t st = g % B_STAGES;
-          mbar_wait(&empty_b[st], ((g / B_STAGES) & 1) ^ 1);
-          mbar_arrive_expect_tx(&full_b[st], B5_STAGE_BYTES);
-          uint8_t *dst = b_smem + st * B5_STAGE_BYTES;
-          const uint32_t row = un.db_row + t * TILE_DB;
-          tma_load_2d(dst, &tmap, 0, (int)row, &full_b[st]);
-          tma_load_2d(dst + A_BYTES, &tmap, 0, (int)(row + 128), &full_b[st]);
-          tma_load_2d(dst + B_BYTES, &tmap_dig, 0, (int)row, &full_b[st]);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================================================================== MMA issuer
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc_u8(TILE_Q, TILE_DB);
-      constexpr uint32_t idesc5 = idesc | (1u << 10);             // B operand signed: u8 weights x s8 digits
-      const uint64_t ac_desc = make_kmajor_sw32_desc(smem_u32(aconst));
-      uint32_t g = 0, ul = 0;
-      for (uint32_t u = blockIdx.x; u < n_units; u += gridDim.x, ++ul) {
-        const uint32_t n_tiles = units[u].n_db_tiles & UNIT_TILES_MASK;
-        const uint32_t as = ul & 1;
-        mbar_wait(&full_a[as], (ul >> 1) & 1);
-        const uint32_t a_addr = smem_u32(a_smem + as * A_BYTES);
-        for (uint32_t t = 0; t < n_tiles; ++t, ++g) {
-          const uint32_t st = g % B_STAGES, acc = g & 1;
-          mbar_wait(&full_b[st], (g / B_STAGES) & 1);
-          mbar_wait(&tmem_empty[acc], ((g >> 1) & 1) ^ 1);
-          tc_fence_after();
-          const uint32_t b_addr = smem_u32(b_smem + st * B5_STAGE_BYTES);
-          const uint32_t d = tmem_base + acc * TILE_DB;
-          #pragma unroll
-          for (int k = 0; k < OMVG_DESC_LEN / 32; ++k)
-            umma_i8(d, make_kmajor_sw128_desc(a_addr + k * 32), make_kmajor_sw128_desc(b_addr + k * 32), idesc, k > 0);
-          umma_i8(d, ac_desc, make_kmajor_sw32_desc(b_addr + B_BYTES), idesc5, 1);
-          tc_commit(&empty_b[st]);
-          tc_commit(&tmem_full[acc]);
-        }
-        tc_commit(&empty_a[as]);
-      }
-    }
-  } else {
-    // ===================================================================== epilogue (8 * NSPLIT warps)
-    const uint32_t e = warp - 2;
-    const uint32_t wg = e / (4 * NSPLIT);                 // accumulator / tile parity served by this warp
-    const uint32_t part = (e % (4 * NSPLIT)) >> 2;        // which 256/NSPLIT-column part of the accumulator
-    const uint32_t quarter = warp & 3;                    // TMEM lane quarter this warp may access
-    const uint32_t row_in_tile = quarter * 32 + lane;
-    constexpr uint32_t NCH = 8 / NSPLIT;                  // 32-column chunks per warp and tile
-    const uint32_t c0 = part * NCH;
-    uint32_t g = 0, ul = 0;
-    for (uint32_t u = blockIdx.x; u < n_units; u += gridDim.x, ++ul) {
-      const Unit un = units[u];
-      const uint32_t n_tiles = un.n_db_tiles & UNIT_TILES_MASK, gdiv = (un.n_db_tiles >> 20) & 0x7FFu;
-      int k1 = KEY_MIN, k2 = KEY_MIN;
-      for (uint32_t t = 0; t < n_tiles; ++t, ++g) {
-        if ((g & 1) != wg) continue;
-        const uint32_t acc = wg;
-        mbar_wait(&tmem_full[acc], (g >> 1) & 1);        // accumulator complete
-        tc_fence_after();
-        const uint32_t taddr = tmem_base + ((quarter * 32) << 16) + acc * TILE_DB + c0 * 32;
-        const uint32_t chunk0 = t * 8 + c0;
-        int32_t ra[32], rb[32];
-        tmem_ld_32x32(taddr, ra);
-        #pragma unroll
-        for (uint32_t c = 0; c < NCH; c += 2) {
-          tmem_ld_wait_dep(ra);
-          tmem_ld_32x32(taddr + (c + 1) * 32, rb);
-          if (!DRAIN_ONLY) chunk_max(ra, (int)(gdiv <= 1 ? chunk0 + c : (chunk0 + c) / gdiv), k1, k2);
-          tmem_ld_wait_dep(rb);
-          if (c + 2 < NCH) tmem_ld_32x32(taddr + (c + 2) * 32, ra);
-          if (!DRAIN_ONLY) chunk_max(rb, (int)(gdiv <= 1 ? chunk0 + c + 1 : (chunk0 + c + 1) / gdiv), k1, k2);
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tmem_empty[acc]);
-      }
-      // merge the partial top-2 lists of the 2 * NSPLIT warps of a row (disjoint chunks) and store
-      int2 *mb = merge + (ul & 1) * NMERGE * TILE_Q;
-      const uint32_t slot = wg * NSPLIT + part;            // slot 0 merges
-      if (slot) mb[(slot - 1) * TILE_Q + row_in_tile] = make_int2(k1, k2);
-      asm volatile("bar.sync 1, %0;" :: "n"(256 * NSPLIT) : "memory");
-      if (slot == 0) {
-        #pragma unroll
-        for (int sI = 0; sI < NMERGE; ++sI) {
-          const int2 o = mb[sI * TILE_Q + row_in_tile];
-          const int lo = min(k1, o.x);
-          k1 = max(k1, o.x);
-          k2 = max(lo, max(k2, o.y));
-        }
-        k12[(size_t)un.out_off + row_in_tile] = make_int2(k1, k2);
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) tmem_dealloc(tmem_base, 512);
-}
-
-
 // --------------------------------------------------------------------------------- two query tiles per database tile
-// match_dig_kernel streams the whole database image through every CTA once per 128 queries: 40 KB per 640 tensor
-// cycles and SM = 18 TB/s of L2 -> SM traffic at full rate, which the L2 does not deliver (the TMA + MMA skeleton
-// WITHOUT any epilogue runs at 61-69 % tensor pipe).  Here one CTA keeps TWO query tiles (256 queries) resident and
-// multiplies both with every database tile it loads: accumulator 0 = queries 0-127, accumulator 1 = queries
-// 128-255, which are at the same time the two halves of the TMEM double buffer (the epilogue of accumulator 0 runs
-// under the MMAs of accumulator 1 and vice versa).  L2 -> SM bytes per MMA halve.  Same keys, same finalize pass.
+// Streaming the whole database image through a CTA once per 128 queries costs 40 KB per 640 tensor cycles and SM =
+// 18 TB/s of L2 -> SM traffic at full rate, which the L2 does not deliver (such a TMA + MMA skeleton WITHOUT any
+// epilogue runs at 61-69 % tensor pipe).  So one CTA keeps TWO query tiles (256 queries) resident and multiplies both
+// with every database tile it loads: accumulator 0 = queries 0-127, accumulator 1 = queries 128-255, which are at the
+// same time the two halves of the TMEM double buffer (the epilogue of accumulator 0 runs under the MMAs of accumulator
+// 1 and vice versa).  NSPLIT = 2 epilogue warps per TMEM lane quarter and accumulator, each draining half the columns.
 constexpr int A2_BYTES = 2 * A_BYTES;                            // 32 KB: two query tiles
 constexpr int B2_STAGES = 3;
+constexpr int NSPLIT = 2;
+constexpr int DIG2_THREADS = 64 + 256 * NSPLIT;                  // TMA warp, MMA warp, 8 * NSPLIT epilogue warps
+constexpr int DIG2_SMEM_BYTES = A_STAGES * A2_BYTES + B2_STAGES * B5_STAGE_BYTES + ACONST_BYTES + 1024 /*align slack*/ + 2 * 2 * TILE_Q * 8 /*merge*/ + 256 /*barriers*/;
 constexpr uint32_t UNIT_TWO = 0x80000000u;                       // Unit.n_db_tiles bit 31: the super-tile has a second query tile
-template <int NSPLIT> constexpr int smem6_bytes() {
-  return A_STAGES * A2_BYTES + B2_STAGES * B5_STAGE_BYTES + ACONST_BYTES + 1024 /*align slack*/ + 2 * 2 * TILE_Q * 8 /*merge*/ + 256 /*barriers*/;
-}
 
-template <int NSPLIT, bool DRAIN_ONLY>
-__global__ void __launch_bounds__(64 + 256 * NSPLIT, 1)
+__global__ void __launch_bounds__(DIG2_THREADS, 1)
 match_dig2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_dig,
                   const Unit *__restrict__ units, uint32_t n_units, int2 *__restrict__ k12) {
   extern __shared__ uint8_t smem_raw[];
@@ -491,7 +339,7 @@ match_dig2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
   uint8_t *a_smem = smem;                                        // [A_STAGES][2 x 16 KB]
   uint8_t *b_smem = smem + A_STAGES * A2_BYTES;                  // [B2_STAGES][32 KB descriptors + 8 KB digits]
   uint8_t *aconst = b_smem + B2_STAGES * B5_STAGE_BYTES;         // [128][32 B] constant weights
-  int2 *merge = reinterpret_cast<int2 *>(aconst + ACONST_BYTES); // [2 accumulators][2][128] (NSPLIT == 2 only)
+  int2 *merge = reinterpret_cast<int2 *>(aconst + ACONST_BYTES); // [2 accumulators][2][128]
   uint64_t *bars = reinterpret_cast<uint64_t *>(merge + 2 * 2 * TILE_Q);
   uint64_t *full_a = bars, *empty_a = bars + 2, *full_b = bars + 4, *empty_b = bars + 8;
   uint64_t *tmem_full = bars + 12, *tmem_empty = bars + 14;
@@ -599,7 +447,7 @@ match_dig2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
         for (uint32_t c = 0; c < NCH; c += 2) {
           tmem_ld_wait_dep(ra);
           tmem_ld_32x32(taddr + (c + 1) * 32, rb);
-          if (!DRAIN_ONLY) chunk_max(ra, (int)(gdiv <= 1 ? chunk0 + c : (chunk0 + c) / gdiv), k1, k2);
+          chunk_max(ra, (int)(gdiv <= 1 ? chunk0 + c : (chunk0 + c) / gdiv), k1, k2);
           tmem_ld_wait_dep(rb);
           if (c + 2 < NCH) tmem_ld_32x32(taddr + (c + 2) * 32, ra);
           else {                                             // every column of the accumulator is in registers: hand it back
@@ -607,15 +455,14 @@ match_dig2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
             __syncwarp();
             if (lane == 0) mbar_arrive(&tmem_empty[wg]);
           }
-          if (!DRAIN_ONLY) chunk_max(rb, (int)(gdiv <= 1 ? chunk0 + c + 1 : (chunk0 + c + 1) / gdiv), k1, k2);
+          chunk_max(rb, (int)(gdiv <= 1 ? chunk0 + c + 1 : (chunk0 + c + 1) / gdiv), k1, k2);
         }
       }
-      if (NSPLIT == 2) {                                   // merge the two column parts of this accumulator
-        int2 *mb = merge + (wg * 2 + (um & 1)) * TILE_Q; ++um;
-        if (part) mb[row_in_tile] = make_int2(k1, k2);
-        if (wg == 0) asm volatile("bar.sync 1, 256;" ::: "memory"); else asm volatile("bar.sync 2, 256;" ::: "memory");
-        if (part == 0) { const int2 o = mb[row_in_tile]; const int lo = min(k1, o.x); k1 = max(k1, o.x); k2 = max(lo, max(k2, o.y)); }
-      }
+      // merge the two column parts of this accumulator
+      int2 *mb = merge + (wg * 2 + (um & 1)) * TILE_Q; ++um;
+      if (part) mb[row_in_tile] = make_int2(k1, k2);
+      if (wg == 0) asm volatile("bar.sync 1, 256;" ::: "memory"); else asm volatile("bar.sync 2, 256;" ::: "memory");
+      if (part == 0) { const int2 o = mb[row_in_tile]; const int lo = min(k1, o.x); k1 = max(k1, o.x); k2 = max(lo, max(k2, o.y)); }
       if (part == 0) k12[(size_t)un.out_off + wg * TILE_Q + row_in_tile] = make_int2(k1, k2);
     }
   }
@@ -626,210 +473,12 @@ match_dig2_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constan
 }
 
 
-// --------------------------------------------------------------------------------- CTA pair (tcgen05 cta_group::2)
-// match_dig2_kernel is bound by shared-memory bandwidth: every SS-mode MMA re-reads A (4 KB) and B (8 KB) from shared
-// memory per 128 tensor cycles, next to the TMA writes.  Here two CTAs of a cluster (one TPC) run ONE M256 N256 K32 MMA
-// per K-slice: CTA r holds query rows [256 r, 256 r + 256) of a 512-query super-tile (two A tiles, as before) and HALF of
-// every database tile (128 of its 256 rows + their digits); the tensor cores exchange the B halves over the pair link,
-// so each SM reads 4 KB + 4 KB per MMA and receives half the TMA bytes.  Only CTA 0 issues MMAs; both load, both drain
-// their own TMEM.  Barrier ownership: full_a / full_b / tmem_empty live in CTA 0 (TMA of CTA 1 completes on them through
-// the peer-masked address, epilogue warps of both CTAs arrive remotely); empty_a / empty_b / tmem_full exist in both
-// CTAs and are signalled by tcgen05.commit ... multicast.
-constexpr uint32_t PEER_MASK = 0xFEFFFFFFu;                       // shared::cluster address of the same offset in CTA 0 of the pair
-constexpr int B3_STAGES = 6;
-constexpr int B3_STAGE_BYTES = A_BYTES + TILE_Q * DIG_LEN;       // 16 KB descriptors + 4 KB digits: half a database tile
-template <int NSPLIT> constexpr int smem7_bytes() {
-  return A_STAGES * A2_BYTES + B3_STAGES * B3_STAGE_BYTES + ACONST_BYTES + 1024 /*align slack*/ + 2 * 2 * TILE_Q * 8 /*merge*/ + 512 /*barriers*/;
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// data into this CTA's shared memory, completion bytes on CTA 0's barrier at the same offset
-__device__ __forceinline__ void tma_load_2d_2sm(void *smem_dst, const void *tmap, int x, int y, uint64_t *bar) {
-  asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-               :: "r"(smem_u32(smem_dst)), "l"(tmap), "r"(smem_u32(bar) & PEER_MASK), "r"(x), "r"(y) : "memory");
-}
-__device__ __forceinline__ void tmem_alloc2(uint32_t *smem_dst, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(smem_dst)), "r"(cols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(taddr), "r"(cols) : "memory");
-}
-// one arrival on the barrier at this offset in BOTH CTAs when all MMAs issued so far have finished
-__device__ __forceinline__ void tc_commit2(uint64_t *bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               :: "r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void umma_i8_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile("{ .reg .pred p; setp.ne.b32 p, %4, 0; tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p; }"
-               :: "r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cta0(uint64_t *bar) {
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" :: "r"(smem_u32(bar) & PEER_MASK) : "memory");
-}
-
-// Unit.n_db_tiles for this kernel: tiles | (rows per group / 32) << 20 (9 bits) | valid 128-query tiles (1..4) << 29
-template <int NSPLIT, bool DRAIN_ONLY>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + 256 * NSPLIT, 1)
-match_dig3_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_dig,
-                  const Unit *__restrict__ units, uint32_t n_units, int2 *__restrict__ k12) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t *a_smem = smem;                                        // [A_STAGES][2 x 16 KB]
-  uint8_t *b_smem = smem + A_STAGES * A2_BYTES;                  // [B3_STAGES][16 KB descriptors + 4 KB digits]
-  uint8_t *aconst = b_smem + B3_STAGES * B3_STAGE_BYTES;         // [128][32 B] constant weights
-  int2 *merge = reinterpret_cast<int2 *>(aconst + ACONST_BYTES); // [2 accumulators][2][128] (NSPLIT == 2 only)
-  uint64_t *bars = reinterpret_cast<uint64_t *>(merge + 2 * 2 * TILE_Q);
-  uint64_t *full_a = bars, *empty_a = bars + 2, *full_b = bars + 4, *empty_b = bars + 4 + B3_STAGES;
-  uint64_t *tmem_full = bars + 4 + 2 * B3_STAGES, *tmem_empty = tmem_full + 2;
-  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(tmem_empty + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const uint32_t cluster_id = blockIdx.x >> 1, n_clusters = gridDim.x >> 1;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap); prefetch_tmap(&tmap_dig);
-    for (int i = 0; i < A_STAGES; ++i) { mbar_init(&full_a[i], 1); mbar_init(&empty_a[i], 1); }
-    for (int i = 0; i < B3_STAGES; ++i) { mbar_init(&full_b[i], 1); mbar_init(&empty_b[i], 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 2 * 4 * NSPLIT); }
-    fence_barrier_init();
-  }
-  for (int i = threadIdx.x; i < ACONST_BYTES / 16; i += blockDim.x)
-    reinterpret_cast<uint4 *>(aconst)[i] = make_uint4(0xFFFFFF01u, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
-  fence_proxy_async();
-  if (warp == 2) tmem_alloc2(tmem_slot, 512);
-  tc_fence_before();
-  cluster_sync_all();                                            // barriers of both CTAs initialised before any remote arrival
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ===================================================================== TMA producer (both CTAs)
-    if (lane == 0) {
-      uint32_t g = 0, ul = 0;
-      for (uint32_t u = cluster_id; u < n_units; u += n_clusters, ++ul) {
-        const Unit un = units[u];
-        const uint32_t as = ul & 1, n_tiles = un.n_db_tiles & UNIT_TILES_MASK;
-        mbar_wait(&empty_a[as], ((ul >> 1) & 1) ^ 1);
-        if (rank == 0) mbar_arrive_expect_tx(&full_a[as], 2 * A2_BYTES);
-        const uint32_t qr = un.q_row + rank * 2 * TILE_Q;
-        tma_load_2d_2sm(a_smem + as * A2_BYTES, &tmap, 0, (int)qr, &full_a[as]);
-        tma_load_2d_2sm(a_smem + as * A2_BYTES + A_BYTES, &tmap, 0, (int)(qr + TILE_Q), &full_a[as]);
-        for (uint32_t t = 0; t < n_tiles; ++t, ++g) {
-          const uint32_t st = g % B3_STAGES;
-          mbar_wait(&empty_b[st], ((g / B3_STAGES) & 1) ^ 1);
-          if (rank == 0) mbar_arrive_expect_tx(&full_b[st], 2 * B3_STAGE_BYTES);
-          uint8_t *dst = b_smem + st * B3_STAGE_BYTES;
-          const uint32_t row = un.db_row + t * TILE_DB + rank * TILE_Q;     // this CTA's half of the database tile
-          tma_load_2d_2sm(dst, &tmap, 0, (int)row, &full_b[st]);
-          tma_load_2d_2sm(dst + A_BYTES, &tmap_dig, 0, (int)row, &full_b[st]);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================================================================== MMA issuer (CTA 0 only)
-    if (lane == 0 && rank == 0) {
-      constexpr uint32_t idesc = make_idesc_u8(2 * TILE_Q, TILE_DB);
-      constexpr uint32_t idesc5 = idesc | (1u << 10);             // B operand signed: u8 weights x s8 digits
-      const uint64_t ac_desc = make_kmajor_sw32_desc(smem_u32(aconst));
-      uint32_t g = 0, ul = 0, cnt[2] = {0, 0};
-      for (uint32_t u = cluster_id; u < n_units; u += n_clusters, ++ul) {
-        const uint32_t ndt = units[u].n_db_tiles;
-        const uint32_t n_tiles = ndt & UNIT_TILES_MASK, nh = (ndt >> 29) >= 2 ? 2u : 1u;
-        const uint32_t as = ul & 1;
-        mbar_wait(&full_a[as], (ul >> 1) & 1);
-        const uint32_t a_addr = smem_u32(a_smem + as * A2_BYTES);
-        for (uint32_t t = 0; t < n_tiles; ++t, ++g) {
-          const uint32_t st = g % B3_STAGES;
-          mbar_wait(&full_b[st], (g / B3_STAGES) & 1);
-          const uint32_t b_addr = smem_u32(b_smem + st * B3_STAGE_BYTES);
-          const uint64_t dg_desc = make_kmajor_sw32_desc(b_addr + A_BYTES);
-          for (uint32_t h = 0; h < nh; ++h) {
-            mbar_wait(&tmem_empty[h], (cnt[h] & 1) ^ 1);
-            tc_fence_after();
-            const uint32_t d = tmem_base + h * TILE_DB;
-            #pragma unroll
-            for (int k = 0; k < OMVG_DESC_LEN / 32; ++k)
-              umma_i8_2sm(d, make_kmajor_sw128_desc(a_addr + h * A_BYTES + k * 32), make_kmajor_sw128_desc(b_addr + k * 32), idesc, k > 0);
-            umma_i8_2sm(d, ac_desc, dg_desc, idesc5, 1);
-            tc_commit2(&tmem_full[h]);
-            ++cnt[h];
-          }
-          tc_commit2(&empty_b[st]);
-        }
-        tc_commit2(&empty_a[as]);
-      }
-    }
-  } else {
-    // ===================================================================== epilogue (8 * NSPLIT warps, both CTAs)
-    const uint32_t e = warp - 2;
-    const uint32_t wg = e / (4 * NSPLIT);                 // accumulator = query tile 2 * rank + wg of the super-tile
-    const uint32_t part = (e % (4 * NSPLIT)) >> 2;
-    const uint32_t quarter = warp & 3;
-    const uint32_t row_in_tile = quarter * 32 + lane;
-    constexpr uint32_t NCH = 8 / NSPLIT;
-    const uint32_t c0 = part * NCH;
-    uint32_t cnt = 0, um = 0;
-    for (uint32_t u = cluster_id; u < n_units; u += n_clusters) {
-      const Unit un = units[u];
-      const uint32_t nvt = un.n_db_tiles >> 29;
-      if (wg == 1 && nvt < 2) continue;                   // accumulator 1 is not used by this super-tile (in either CTA)
-      const bool valid = 2 * rank + wg < nvt;             // this query tile holds real rows
-      const uint32_t n_tiles = un.n_db_tiles & UNIT_TILES_MASK, gdiv = (un.n_db_tiles >> 20) & 0x1FFu;
-      int k1 = KEY_MIN, k2 = KEY_MIN;
-      for (uint32_t t = 0; t < n_tiles; ++t, ++cnt) {
-        mbar_wait(&tmem_full[wg], cnt & 1);
-        tc_fence_after();
-        if (!valid) {                                     // padding tile: just hand the accumulator back
-          tc_fence_before(); __syncwarp();
-          if (lane == 0) mbar_arrive_cta0(&tmem_empty[wg]);
-          continue;
-        }
-        const uint32_t taddr = tmem_base + ((quarter * 32) << 16) + wg * TILE_DB + c0 * 32;
-        const uint32_t chunk0 = t * 8 + c0;
-        int32_t ra[32], rb[32];
-        tmem_ld_32x32(taddr, ra);
-        #pragma unroll
-        for (uint32_t c = 0; c < NCH; c += 2) {
-          tmem_ld_wait_dep(ra);
-          tmem_ld_32x32(taddr + (c + 1) * 32, rb);
-          if (!DRAIN_ONLY) chunk_max(ra, (int)(gdiv <= 1 ? chunk0 + c : (chunk0 + c) / gdiv), k1, k2);
-          tmem_ld_wait_dep(rb);
-          if (c + 2 < NCH) tmem_ld_32x32(taddr + (c + 2) * 32, ra);
-          else {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cta0(&tmem_empty[wg]);
-          }
-          if (!DRAIN_ONLY) chunk_max(rb, (int)(gdiv <= 1 ? chunk0 + c + 1 : (chunk0 + c + 1) / gdiv), k1, k2);
-        }
-      }
-      if (!valid) continue;                               // (uniform over the warps of this accumulator)
-      if (NSPLIT == 2) {
-        int2 *mb = merge + (wg * 2 + (um & 1)) * TILE_Q; ++um;
-        if (part) mb[row_in_tile] = make_int2(k1, k2);
-        if (wg == 0) asm volatile("bar.sync 1, 256;" ::: "memory"); else asm volatile("bar.sync 2, 256;" ::: "memory");
-        if (part == 0) { const int2 o = mb[row_in_tile]; const int lo = min(k1, o.x); k1 = max(k1, o.x); k2 = max(lo, max(k2, o.y)); }
-      }
-      if (part == 0) k12[(size_t)un.out_off + (2 * rank + wg) * TILE_Q + row_in_tile] = make_int2(k1, k2);
-    }
-  }
-
-  tc_fence_before();
-  cluster_sync_all();                                     // the peer may still be reading this CTA's shared memory / TMEM
-  if (warp == 2) tmem_dealloc2(tmem_base, 512);
-}
-
 // --------------------------------------------------------------------------------- finalize
 struct PairInfo { uint32_t db_row0, db_count, db_group, q_row0, q_count; uint32_t unit0; uint64_t out_off; int32_t db_c0; int32_t pad_; };
 
 // expand the per-pair table into the (pair, 128-query tile) work units on the device (one block per pair)
-// q_tiles = 1: one unit per 128 queries; q_tiles = 2 (match_dig2_kernel): one unit per 256 queries, UNIT_TWO set when the
-// second query tile holds real rows
-// q_tiles = 4 (match_dig3_kernel): one unit per 512 queries, the number of query tiles with real rows in bits 29-31
+// q_tiles = 1 (match_tc_kernel): one unit per 128 queries; q_tiles = 2 (match_dig2_kernel): one unit per 256 queries,
+// UNIT_TWO set when the second query tile holds real rows
 __global__ void expand_units_kernel(const PairInfo *__restrict__ pairs, Unit *__restrict__ units, uint32_t q_tiles) {
   const PairInfo P = pairs[blockIdx.x];
   const uint32_t rows = TILE_Q * q_tiles;
@@ -837,7 +486,6 @@ __global__ void expand_units_kernel(const PairInfo *__restrict__ pairs, Unit *__
   for (uint32_t t = threadIdx.x; t < qt; t += blockDim.x) {
     uint32_t flags = 0;
     if (q_tiles == 2 && P.q_count - t * rows > TILE_Q) flags = UNIT_TWO;
-    if (q_tiles == 4) flags = min(4u, (P.q_count - t * rows + TILE_Q - 1) / TILE_Q) << 29;
     units[P.unit0 + t] = Unit{P.q_row0 + t * rows, P.db_row0, dt | ((P.db_group / 32) << 20) | flags, (uint32_t)(P.out_off + t * rows)};
   }
 }
@@ -879,7 +527,7 @@ __device__ __forceinline__ void warp_rescan(const uint8_t *__restrict__ desc, co
 
 constexpr int FIN_THREADS = 256;
 // DIG = false: keys of match_tc_kernel (exact d1, exact bound ub2).
-// DIG = true : keys of match_dig_kernel.  A = key >> 8 is the chunk maximum of acc = q.b - h + c0, so the best column
+// DIG = true : keys of match_dig2_kernel.  A = key >> 8 is the chunk maximum of acc = q.b - h + c0, so the best column
 // of that chunk has distance  D - 1 or D,  D = |q|^2 - 2 A + 2 c0  (parity of |b|^2 unknown).  Then
 //   * A1 > A2: the nearest neighbour lies in the chunk (group) of A1 — every other column has acc <= A2 <= A1 - 1, i.e.
 //     distance >= D1 + 1; its exact distance and index come from the group re-scan as before.
@@ -1280,9 +928,8 @@ struct omvg_match_ctx {
   uint8_t *d_desc = nullptr; int32_t *d_norm = nullptr, *d_ckey = nullptr;
   uint32_t *d_img_row0 = nullptr, *d_img_count = nullptr, *d_img_group = nullptr, *d_row_img = nullptr;
   bool uploaded = false, prepared = false;
-  CUtensorMap tmap, tmap_dig, tmap_dig128;   // digits: 256-row boxes (one CTA per tile) and 128-row boxes (CTA pair)
-  int max_clusters = 0;
-  // fifth-slice kernel (match_dig_kernel): 32 signed digits per arena row, per-image offset c0, eligibility
+  CUtensorMap tmap, tmap_dig;   // descriptors: 128-row boxes; digits: 256-row boxes (one database tile)
+  // fifth-slice kernel (match_dig2_kernel): 32 signed digits per arena row, per-image offset c0, eligibility
   uint4 *d_dig = nullptr; int32_t *d_img_c0 = nullptr; int2 *d_hmm = nullptr; std::vector<int32_t> c0; bool use_dig = false;
   // run state
   int2 *d_k12 = nullptr; size_t k12_cap = 0;           // in int2 elements
@@ -1327,11 +974,6 @@ int make_tmap(omvg_match_ctx *c) {
                                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B,
                                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r2 != CUDA_SUCCESS) return fail(OMVG_E_CUDA, "cuTensorMapEncodeTiled (digits) failed (%d)", (int)r2);
-  const cuuint32_t dbox2[2] = {DIG_LEN, TILE_Q};
-  const CUresult r3 = ((encode_tiled_fn)fn)(&c->tmap_dig128, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, c->d_dig, ddims, dstrides, dbox2, estr,
-                                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B,
-                                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r3 != CUDA_SUCCESS) return fail(OMVG_E_CUDA, "cuTensorMapEncodeTiled (digits, 128 rows) failed (%d)", (int)r3);
   return OMVG_OK;
 }
 
@@ -1369,9 +1011,7 @@ int run_batch(omvg_match_ctx *c, const uint32_t *pi, const uint32_t *pj, uint64_
               std::vector<Unit> &units, std::vector<PairInfo> &pinfo) {
   units.clear(); pinfo.clear();
   size_t out = 0, n_units = 0;
-  const bool use_dig2 = c->use_dig && !getenv("OMVG_MATCH_M128");   // A/B: one query tile per CTA pass (match_dig_kernel)
-  bool use_dig3 = use_dig2 && c->max_clusters > 0 && getenv("OMVG_MATCH_2SM") != nullptr;   // CTA pair, tcgen05 cta_group::2
-  if (use_dig3) for (uint64_t p = p0; p < p1; ++p) if (c->group[pi[p]] / 32 >= 512) { use_dig3 = false; break; }
+  const uint32_t q_tiles = c->use_dig ? 2 : 1;            // query tiles per unit: match_dig2_kernel takes two
   for (uint64_t p = p0; p < p1; ++p) {
     const uint32_t I = pi[p], J = pj[p];
     PairInfo P{}; P.db_row0 = c->row0[I]; P.db_count = c->counts[I]; P.db_group = c->group[I]; P.db_c0 = c->c0.empty() ? 0 : c->c0[I];
@@ -1382,7 +1022,7 @@ int run_batch(omvg_match_ctx *c, const uint32_t *pi, const uint32_t *pj, uint64_
     pinfo.push_back(P);
     if (!active) continue;
     const uint32_t qt = (P.q_count + TILE_Q - 1) / TILE_Q;
-    pinfo.back().unit0 = (uint32_t)n_units; n_units += use_dig3 ? (qt + 3) / 4 : (use_dig2 ? (qt + 1) / 2 : qt);
+    pinfo.back().unit0 = (uint32_t)n_units; n_units += (qt + q_tiles - 1) / q_tiles;
     out += size_t(qt) * TILE_Q;
   }
   if (out > 0xffffffffull) return fail(OMVG_E_ARG, "batch too large");
@@ -1398,34 +1038,12 @@ int run_batch(omvg_match_ctx *c, const uint32_t *pi, const uint32_t *pj, uint64_
   }
   OMVG_CUDA(cudaMemcpyAsync(c->d_pairs, pinfo.data(), nb * sizeof(PairInfo), cudaMemcpyHostToDevice, c->stream));
   if (n_units) {
-    expand_units_kernel<<<nb, 64, 0, c->stream>>>(c->d_pairs, c->d_units, use_dig3 ? 4u : (use_dig2 ? 2u : 1u)); OMVG_CUDA(cudaGetLastError()); c->launches++;
+    expand_units_kernel<<<nb, 64, 0, c->stream>>>(c->d_pairs, c->d_units, q_tiles); OMVG_CUDA(cudaGetLastError()); c->launches++;
     const uint32_t grid = (uint32_t)std::min<size_t>(n_units, (size_t)c->n_sms);
     cudaEvent_t e0 = get_event(c), e1 = get_event(c);
     OMVG_CUDA(cudaEventRecord(e0, c->stream));
-    // OMVG_MATCH_DRAIN_ONLY=1 (measurement aid, results are garbage): epilogue reads TMEM but does no arithmetic
-    static const bool drain_only = getenv("OMVG_MATCH_DRAIN_ONLY") != nullptr;
-    const int nsplit = getenv("OMVG_MATCH_NSPLIT") ? atoi(getenv("OMVG_MATCH_NSPLIT")) : MATCH_NSPLIT_DEFAULT;   // epilogue warps per lane quarter and accumulator
-    if (use_dig3) {
-      const uint32_t grid3 = 2 * (uint32_t)std::min<size_t>(n_units, (size_t)c->max_clusters);
-      if (nsplit == 2) { if (drain_only) match_dig3_kernel<2, true><<<grid3, 64 + 512, smem7_bytes<2>(), c->stream>>>(c->tmap, c->tmap_dig128, c->d_units, (uint32_t)n_units, c->d_k12);
-                         else match_dig3_kernel<2, false><<<grid3, 64 + 512, smem7_bytes<2>(), c->stream>>>(c->tmap, c->tmap_dig128, c->d_units, (uint32_t)n_units, c->d_k12); }
-      else             { if (drain_only) match_dig3_kernel<1, true><<<grid3, 64 + 256, smem7_bytes<1>(), c->stream>>>(c->tmap, c->tmap_dig128, c->d_units, (uint32_t)n_units, c->d_k12);
-                         else match_dig3_kernel<1, false><<<grid3, 64 + 256, smem7_bytes<1>(), c->stream>>>(c->tmap, c->tmap_dig128, c->d_units, (uint32_t)n_units, c->d_k12); }
-    }
-    else if (use_dig2) {
-      if (nsplit == 2) { if (drain_only) match_dig2_kernel<2, true><<<grid, 64 + 512, smem6_bytes<2>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12);
-                         else match_dig2_kernel<2, false><<<grid, 64 + 512, smem6_bytes<2>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12); }
-      else             { if (drain_only) match_dig2_kernel<1, true><<<grid, 64 + 256, smem6_bytes<1>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12);
-                         else match_dig2_kernel<1, false><<<grid, 64 + 256, smem6_bytes<1>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12); }
-    }
-    else if (c->use_dig) {
-      if (nsplit == 2) { if (drain_only) match_dig_kernel<2, true><<<grid, 64 + 512, smem5_bytes<2>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12);
-                         else match_dig_kernel<2, false><<<grid, 64 + 512, smem5_bytes<2>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12); }
-      else             { if (drain_only) match_dig_kernel<1, true><<<grid, 64 + 256, smem5_bytes<1>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12);
-                         else match_dig_kernel<1, false><<<grid, 64 + 256, smem5_bytes<1>(), c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12); }
-    }
-    else if (drain_only) match_tc_kernel<1><<<grid, TC_THREADS, SMEM_BYTES, c->stream>>>(c->tmap, c->d_ckey, c->d_units, (uint32_t)n_units, c->d_k12);
-    else match_tc_kernel<0><<<grid, TC_THREADS, SMEM_BYTES, c->stream>>>(c->tmap, c->d_ckey, c->d_units, (uint32_t)n_units, c->d_k12);
+    if (c->use_dig) match_dig2_kernel<<<grid, DIG2_THREADS, DIG2_SMEM_BYTES, c->stream>>>(c->tmap, c->tmap_dig, c->d_units, (uint32_t)n_units, c->d_k12);
+    else match_tc_kernel<<<grid, TC_THREADS, SMEM_BYTES, c->stream>>>(c->tmap, c->d_ckey, c->d_units, (uint32_t)n_units, c->d_k12);
     OMVG_CUDA(cudaGetLastError());
     OMVG_CUDA(cudaEventRecord(e1, c->stream));
     c->pending.emplace_back(e0, e1); c->tc_launches++; c->launches++;
@@ -1479,28 +1097,8 @@ int omvg_match_create(omvg_match_ctx **out, int device) {
   OMVG_CUDA(cudaSetDevice(device));
   omvg_match_ctx *c = new omvg_match_ctx; c->device = device; c->n_sms = n_sms;
   OMVG_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-  OMVG_CUDA(cudaFuncSetAttribute(match_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-  OMVG_CUDA(cudaFuncSetAttribute(match_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig3_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem7_bytes<1>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig3_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem7_bytes<1>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig3_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem7_bytes<2>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig3_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem7_bytes<2>()));
-  { // how many CTA pairs can be resident at once (a GPC with an odd number of usable SMs leaves one SM without a partner)
-    cudaLaunchConfig_t cfg{}; cfg.gridDim = dim3(2 * n_sms); cfg.blockDim = dim3(64 + 512); cfg.dynamicSmemBytes = smem7_bytes<2>();
-    cudaLaunchAttribute at{}; at.id = cudaLaunchAttributeClusterDimension; at.val.clusterDim.x = 2; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
-    cfg.attrs = &at; cfg.numAttrs = 1;
-    int ncl = 0;
-    if (cudaOccupancyMaxActiveClusters(&ncl, match_dig3_kernel<2, false>, &cfg) != cudaSuccess) { cudaGetLastError(); ncl = 0; }
-    c->max_clusters = ncl;
-  }
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig2_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem6_bytes<1>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig2_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem6_bytes<1>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig2_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem6_bytes<2>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig2_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem6_bytes<2>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem5_bytes<1>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem5_bytes<1>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem5_bytes<2>()));
-  OMVG_CUDA(cudaFuncSetAttribute(match_dig_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem5_bytes<2>()));
+  OMVG_CUDA(cudaFuncSetAttribute(match_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+  OMVG_CUDA(cudaFuncSetAttribute(match_dig2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DIG2_SMEM_BYTES));
   OMVG_CUDA(cudaMalloc(&c->d_total, sizeof(uint64_t)));
   if (const char *e = getenv("OMVG_MATCH_K12_MB")) c->k12_budget_bytes = size_t(atol(e)) << 20;
   *out = c; return OMVG_OK;
@@ -1675,7 +1273,6 @@ int omvg_match_fetch(omvg_match_ctx *c, const uint64_t **offsets, const uint32_t
 
 uint64_t omvg_match_launch_count(const omvg_match_ctx *c) { return c ? c->launches : 0; }
 int omvg_match_kernel_variant(const omvg_match_ctx *c) { return (!c || !c->prepared) ? 0 : (c->use_dig ? 5 : 4); }
-int omvg_match_max_clusters(const omvg_match_ctx *c) { return c ? c->max_clusters : 0; }
 
 int omvg_match_kernel_time(omvg_match_ctx *c, double *ms, uint64_t *launches, int reset) {
   if (!c) return fail(OMVG_E_ARG, "null ctx");
@@ -1862,7 +1459,7 @@ int omvg_match_debug_top2_tc(omvg_match_ctx *c, uint32_t I, uint32_t J, int32_t 
   if ((rc = ensure(c->d_k12, c->k12_cap, size_t(qt) * TILE_Q))) return rc;
   if ((rc = ensure(c->d_units, c->units_cap, units.size()))) return rc;
   OMVG_CUDA(cudaMemcpyAsync(c->d_units, units.data(), units.size() * sizeof(Unit), cudaMemcpyHostToDevice, c->stream));
-  match_tc_kernel<0><<<std::min<uint32_t>(qt, c->n_sms), TC_THREADS, SMEM_BYTES, c->stream>>>(c->tmap, c->d_ckey, c->d_units, qt, c->d_k12);
+  match_tc_kernel<<<std::min<uint32_t>(qt, c->n_sms), TC_THREADS, SMEM_BYTES, c->stream>>>(c->tmap, c->d_ckey, c->d_units, qt, c->d_k12);
   OMVG_CUDA(cudaGetLastError()); c->launches++;
   int32_t *dd1, *dd2; uint32_t *dg1;
   OMVG_CUDA(cudaMalloc(&dd1, nq * 4)); OMVG_CUDA(cudaMalloc(&dd2, nq * 4)); OMVG_CUDA(cudaMalloc(&dg1, nq * 4));

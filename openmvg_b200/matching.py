@@ -100,9 +100,6 @@ class MatchContext:
         """5 = fifth-K-slice kernel, 4 = key-arithmetic kernel (see omvg_match_kernel_variant)."""
         return int(lib().omvg_match_kernel_variant(self._h))
 
-    def max_clusters(self) -> int:
-        return int(lib().omvg_match_max_clusters(self._h))
-
     def kernel_time(self, reset: bool = True):
         ms = ctypes.c_double(); n = ctypes.c_uint64()
         check(lib().omvg_match_kernel_time(self._h, ctypes.byref(ms), ctypes.byref(n), int(reset)))

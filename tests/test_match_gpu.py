@@ -318,7 +318,7 @@ def test_load_desc_files_equals_in_memory_upload(tmp_path):
             assert np.array_equal(seen[key], m)
 
 
-# ---- the fifth-K-slice kernel (match_dig_kernel) against the key-arithmetic kernel and the oracle
+# ---- the fifth-K-slice kernel (match_dig2_kernel) against the key-arithmetic kernel and the oracle
 def _near_tie_collection(seed):
     """Rows that differ from each other by +-1 in a few elements: distances of 0, 1, 2, ... with both parities of |b|^2,
     so the chunk maxima tie to within the parity and the exact-scan fallbacks of the finalize pass run."""
@@ -357,8 +357,7 @@ def test_fifth_slice_near_ties(matching, seed):
 
 
 def test_kernel_variants_agree(matching, monkeypatch):
-    """Default (fifth slice, two query tiles per database tile) = two epilogue warps per lane quarter = one query tile per
-    database tile = the key-arithmetic kernel."""
+    """Default (fifth slice, two query tiles per database tile) = the key-arithmetic kernel (OMVG_MATCH_TC4) = the oracle."""
     rng = np.random.default_rng(8)
     descs = synth.descriptors(5, [1500, 700, 2300, 33, 900], seed=31)
     descs.append(rng.integers(0, 256, (800, 128), dtype=np.int64).astype(np.uint8))       # |b|^2 ~ 2.8e6: c0 > 0
@@ -367,9 +366,8 @@ def test_kernel_variants_agree(matching, monkeypatch):
     pi = np.concatenate([pi, pj]); pj = np.concatenate([pj, pi[:len(pj)]])
     ooff, oij = ck.oracle_match_collection(descs, pi, pj, 0.8)
     results = []
-    for env in ({}, {"OMVG_MATCH_NSPLIT": "1"}, {"OMVG_MATCH_2SM": "1"}, {"OMVG_MATCH_2SM": "1", "OMVG_MATCH_NSPLIT": "1"}, {"OMVG_MATCH_M128": "1"},
-                {"OMVG_MATCH_M128": "1", "OMVG_MATCH_NSPLIT": "1"}, {"OMVG_MATCH_TC4": "1"}):
-        for k in ("OMVG_MATCH_NSPLIT", "OMVG_MATCH_TC4", "OMVG_MATCH_M128", "OMVG_MATCH_2SM"): monkeypatch.delenv(k, raising=False)
+    for env in ({}, {"OMVG_MATCH_TC4": "1"}):
+        monkeypatch.delenv("OMVG_MATCH_TC4", raising=False)
         for k, v in env.items(): monkeypatch.setenv(k, v)
         ctx = matching.MatchContext(0)
         ctx.load(descs)

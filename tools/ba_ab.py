@@ -17,8 +17,8 @@ for _ in range(5):
 print(json.dumps(dict(device_ms=best["device_ms"], iters=best["iterations"], pcg=best["pcg_iterations"], cost=best["final_cost"], launches=best["kernel_launches"])))
 '''
 cfg = [int(x) for x in sys.argv[1:4]] if len(sys.argv) >= 4 else [1000, 100000, 10]
-variants = [("default (pcg5)", {}), ("pcg3 (4 syncs)", {"OMVG_BA_PCG3": "1"}), ("pcg5 timing", {"OMVG_BA_PCG_TIMING": "1"}), ("pcg4 (2 syncs)", {"OMVG_BA_PCG4": "1"}), ("coarse every step", {"OMVG_BA_COARSE_EVERY": "1"}), ("coarse every 4", {"OMVG_BA_COARSE_EVERY": "4"}),
-            ("pcg3 timing", {"OMVG_BA_PCG_TIMING": "1"}), ("pcg4 timing", {"OMVG_BA_PCG_TIMING": "1", "OMVG_BA_PCG4": "1"}), ("gj timing", {"OMVG_BA_GJ_TIMING": "1"})]
+variants = [("default (pcg5)", {}), ("pcg5 timing", {"OMVG_BA_PCG_TIMING": "1"}), ("coarse every step", {"OMVG_BA_COARSE_EVERY": "1"}), ("coarse every 4", {"OMVG_BA_COARSE_EVERY": "4"}),
+            ("gj timing", {"OMVG_BA_GJ_TIMING": "1"})]
 for name, env in variants:
     e = dict(os.environ); e.update(env)
     p = subprocess.run([sys.executable, "-c", CHILD % (ROOT, *cfg)], capture_output=True, text=True, env=e, timeout=600)

@@ -9,7 +9,7 @@ descs = synth.descriptors(n, 5000, seed=1000)
 pi, pj = synth.exhaustive_pairs(n)
 ctx = matching.MatchContext(0)
 ctx.load(descs)
-print('kernel variant', ctx.kernel_variant(), 'max clusters', ctx.max_clusters())
+print('kernel variant', ctx.kernel_variant())
 for r in range(reps):
     t = time.time(); ctx.run(pi, pj, 0.8); ctx.sync(); dt = time.time() - t
     ms, k = ctx.kernel_time()
