@@ -8,6 +8,7 @@
 // termination decisions from a handful of scalars read back once per LM iteration.
 #include "ba_kernels.cuh"
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include <algorithm>
 #include <cmath>
@@ -74,6 +75,7 @@ struct omvg_ba_ctx {
   DevBuf<unsigned long long> pcg_tim;
   DevBuf<double> corner_rep;
   DevBuf<double> GE;                        // per observation { Einv E'Fc, E'Fc } of the split Schur step
+  DevBuf<unsigned long long> pairs; DevBuf<int> gstart, gblk, gblkT; int nwork = 0;   // pair lists of schur_gather_kernel
   // optional extensions: GCP weights / flags / fixed landmarks, pose-centre priors
   DevBuf<double> obs_w; DevBuf<unsigned char> obs_flags, pt_fixed; DevBuf<unsigned> pt_mask;
   DevBuf<unsigned char> pt_gcp, pt_removed, pt_now; DevBuf<unsigned> rej_bits; DevBuf<unsigned long long> rej_cnt;   // outlier rejection (omvg_ba_reject_outliers)
@@ -369,6 +371,58 @@ int build_structure(omvg_ba_ctx *c) {
   return c->Scc.alloc((size_t)c->nnzb * 36);
 }
 
+// Pair lists of schur_gather_kernel (see pair_fill_kernel).  Work list: the diagonal blocks first (one entry per
+// observation of the camera: the longest lists start first), then the upper off-diagonal blocks row by row, so that the
+// rows in flight share their landmarks' GE records in L2.
+int build_pair_lists(omvg_ba_ctx *c) {
+  int rc;
+  std::vector<int> hp(c->nc + 1), hcols(c->nnzb);
+  OMVG_CUDA(cudaMemcpyAsync(hp.data(), c->rowptr.p, (c->nc + 1) * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  OMVG_CUDA(cudaMemcpyAsync(hcols.data(), c->cols.p, (size_t)c->nnzb * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  OMVG_CUDA(cudaStreamSynchronize(c->stream));
+  auto find = [&](int a, int b) { return (int)(std::lower_bound(hcols.begin() + hp[a], hcols.begin() + hp[a + 1], b) - hcols.begin()); };
+  std::vector<int> wpos(c->nnzb, -1), gblk, gblkT;
+  for (int a = 0; a < c->nc; ++a) { const int e = find(a, a); wpos[e] = (int)gblk.size(); gblk.push_back(e); gblkT.push_back(e); }
+  for (int a = 0; a < c->nc; ++a)
+    for (int e = hp[a]; e < hp[a + 1]; ++e) if (hcols[e] > a) { wpos[e] = (int)gblk.size(); gblk.push_back(e); gblkT.push_back(find(hcols[e], a)); }
+  c->nwork = (int)gblk.size();
+  cudaStream_t s = c->stream;
+  DevBuf<int> d_wpos;
+  if ((rc = upload(c->gblk, gblk.data(), gblk.size(), s)) || (rc = upload(c->gblkT, gblkT.data(), gblkT.size(), s)) || (rc = upload(d_wpos, wpos.data(), wpos.size(), s))) return rc;
+  DevBuf<long long> cnt, offs; DevBuf<unsigned char> tmp;
+  if ((rc = cnt.alloc(c->np + 1)) || (rc = offs.alloc(c->np + 1)) || (rc = c->gstart.alloc(c->nwork + 1))) return rc;
+  pair_count_kernel<<<(c->np + 256) / 256, 256, 0, s>>>(c->pt_start.p, c->pt_single.p, c->obs_pose.p, c->np, cnt.p); LAUNCH_CHECK();
+  size_t tb = 0;
+  OMVG_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, cnt.p, offs.p, c->np + 1, s));
+  if ((rc = tmp.alloc(tb))) return rc;
+  OMVG_CUDA(cub::DeviceScan::ExclusiveSum(tmp.p, tb, cnt.p, offs.p, c->np + 1, s));
+  long long total = 0;
+  OMVG_CUDA(cudaMemcpyAsync(&total, offs.p + c->np, sizeof total, cudaMemcpyDeviceToHost, s));
+  OMVG_CUDA(cudaStreamSynchronize(s));
+  if (total > std::numeric_limits<int>::max()) return fail(OMVG_E_UNSUPPORTED, "%lld camera-pair terms of the Schur complement (at most 2^31 - 1)", total);
+  const int n = (int)total;
+  if (n > 0) {
+    DevBuf<int> k0, k1; DevBuf<unsigned long long> p0;
+    if ((rc = k0.alloc(n)) || (rc = k1.alloc(n)) || (rc = p0.alloc(n)) || (rc = c->pairs.alloc(n))) return rc;
+    pair_fill_kernel<<<(c->np + 255) / 256, 256, 0, s>>>(c->pt_start.p, c->pt_single.p, c->obs_pose.p, c->np, offs.p, Bsr{c->bitmap.p, c->wprefix.p, c->rowptr.p, c->words}, d_wpos.p, k0.p, p0.p); LAUNCH_CHECK();
+    int kbits = 1; while ((1ll << kbits) < c->nwork) ++kbits;
+    size_t sb = 0;
+    OMVG_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sb, k0.p, k1.p, p0.p, c->pairs.p, n, 0, kbits, s));
+    if (sb > tmp.n && (rc = tmp.alloc(sb))) return rc;
+    sb = tmp.n;
+    OMVG_CUDA(cub::DeviceRadixSort::SortPairs(tmp.p, sb, k0.p, k1.p, p0.p, c->pairs.p, n, 0, kbits, s));
+    setup_starts_kernel<<<(unsigned)((n + 256) / 256), 256, 0, s>>>(k1.p, n, c->nwork, c->gstart.p); LAUNCH_CHECK();
+    OMVG_CUDA(cudaStreamSynchronize(s));               // the temporaries are released at the end of this scope
+    c->launches += 2;
+  } else {
+    OMVG_CUDA(cudaMemsetAsync(c->gstart.p, 0, (c->nwork + 1) * sizeof(int), s));
+    OMVG_CUDA(cudaStreamSynchronize(s));
+  }
+  c->launches += 1;
+  if (getenv("OMVG_BA_TIMING")) fprintf(stderr, "[omvg_ba structure] %d upper S blocks, %d pair-list entries (%.1f MB)\n", c->nwork, n, n * 8e-6);
+  return OMVG_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -508,6 +562,8 @@ int omvg_ba_create(omvg_ba_ctx **out, int device, const omvg_ba_problem *P) {
   tm.lap("allocations");
   if ((rc = build_structure(c))) return rc;
   tm.lap("structure");
+  if ((rc = build_pair_lists(c))) return rc;
+  tm.lap("pair lists");
   OMVG_CUDA(cudaStreamWaitEvent(s, c->ev_up, 0));
   setup_gather_xy_kernel<<<(unsigned)((no + 255) / 256), 256, 0, s>>>(c->d_perm.p, reinterpret_cast<const double2 *>(raw_xy.p), raw_w.p, raw_fl.p, no,
                                                                   reinterpret_cast<double2 *>(c->obs_xy.p), c->obs_w.p, c->obs_flags.p); LAUNCH_CHECK();
@@ -613,16 +669,17 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
       lm_diag3_kernel<<<dim3(nb, 3), 256, 0, c->stream>>>(DG, O->min_lm_diagonal, O->max_lm_diagonal, radius); LAUNCH_CHECK(); }
     // ---- reduced camera system
     if (m.pts_free && !c->corner_rep.p) { if ((rc = c->corner_rep.alloc((size_t)CORNER_REPS * (KI * KI + KI)))) return rc; }
-    { Zero4 Z{}; Z.p[0] = c->Scc.p; Z.n[0] = (long long)c->nnzb * 36; Z.p[1] = c->Sci.p; Z.n[1] = (long long)c->Sci.n; Z.p[2] = c->Sii.p; Z.n[2] = (long long)c->Sii.n;
+    { Zero4 Z{}; Z.p[0] = c->Scc.p; Z.n[0] = m.pts_free ? 0 : (long long)c->nnzb * 36;     // (schur_gather_kernel writes all of Scc)
+      Z.p[1] = c->Sci.p; Z.n[1] = (long long)c->Sci.n; Z.p[2] = c->Sii.p; Z.n[2] = (long long)c->Sii.n;
       Z.p[3] = m.pts_free ? c->corner_rep.p : c->rhs.p; Z.n[3] = m.pts_free ? (long long)c->corner_rep.n : 0;     // (rhs is fully written by s_init_kernel)
-      const int nb = (int)std::max<long long>(1, std::min<long long>(4 * c->n_sms, (Z.n[0] + 255) / 256));
+      const long long zmax = std::max(std::max(Z.n[0], Z.n[1]), std::max(Z.n[2], Z.n[3]));
+      const int nb = (int)std::max<long long>(1, std::min<long long>(4 * c->n_sms, (zmax + 255) / 256));
       zero4_kernel<<<dim3(nb, 4), 256, 0, c->stream>>>(Z); LAUNCH_CHECK(); }
     SchurArgs SA{}; SA.r = c->r.p; SA.Jp = c->Jp.p; SA.Jc = c->Jc.p; SA.Ji = c->Ji.p; SA.EtE = c->EtE.p; SA.Etb = c->Etb.p; SA.EtFi = c->EtFi.p; SA.lmD_pt = c->lmD_pt.p; SA.pt_single = c->pt_single.p; SA.FtF = c->FtF.p; SA.FiFi = c->FiFi.p; SA.g_cam = c->g_cam.p; SA.g_intr = c->g_intr.p;
     SA.obs_pose = c->obs_pose.p; SA.obs_intr = c->obs_intr.p; SA.obs_pt = c->obs_pt.p; SA.pt_start = c->pt_start.p; SA.n = c->no; SA.n_poses = c->nc; SA.n_intr = c->ni;
     SA.pts_free = m.pts_free; SA.kiu = c->kiu; SA.bsr = Bsr{c->bitmap.p, c->wprefix.p, c->rowptr.p, c->words}; SA.Scc = c->Scc.p; SA.Sci = c->Sci.p; SA.Sii = c->Sii.p; SA.rhs = c->rhs.p;
     SA.Einv = c->Einv.p; SA.fail = c->fail.p;
     { const int ninit = std::max(std::max(36 * c->nc, 64 * c->ni), c->nred); s_init_kernel<<<(ninit + 255) / 256, 256, 0, c->stream>>>(SA); LAUNCH_CHECK(); }
-    SA.n_points = c->np;
     if (m.pts_free) {
       if (!c->GE.p) { if ((rc = c->GE.alloc(36 * (size_t)c->no))) return rc; }
       { const unsigned sg = (unsigned)((c->no + SCHUR_THREADS - 1) / SCHUR_THREADS);
@@ -638,13 +695,14 @@ int omvg_ba_run(omvg_ba_ctx *c, const omvg_ba_options *O, omvg_ba_summary *sum) 
       }
       LAUNCH_CHECK();
       corner_fold_kernel<<<1, 96, 0, c->stream>>>(c->corner_rep.p, c->obs_intr.p, c->nc, c->ni, c->Sii.p, c->rhs.p); LAUNCH_CHECK(); c->launches++;
-      static const int occ2 = [] { int o = 1; cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, schur_pair_kernel, 256, 0); return std::max(1, o); }();   // (thread-safe: Adjust may run on several host threads)
-      schur_pair_kernel<<<c->n_sms * occ2, 256, 0, c->stream>>>(SA, c->GE.p); LAUNCH_CHECK(); c->launches += 2;
+      schur_gather_kernel<<<(unsigned)(((long long)c->nwork * 32 + GATHER_THREADS - 1) / GATHER_THREADS), GATHER_THREADS, 0, c->stream>>>(
+          c->GE.p, c->gstart.p, reinterpret_cast<const int2 *>(c->pairs.p), c->gblk.p, c->gblkT.p, c->nwork, c->brow.p, c->FtF.p, c->Scc.p); LAUNCH_CHECK();
+      c->launches += 2;
       SA.skip_fast = 1;
     }
+    // the remaining landmarks (several intrinsic groups, more than 32 observations) add to the gathered Scc: after it
     if (!m.pts_free || c->n_slow > 0) { schur_kernel<<<(unsigned)((c->no + SCHUR_THREADS - 1) / SCHUR_THREADS), SCHUR_THREADS, 0, c->stream>>>(SA); LAUNCH_CHECK(); }
-    mirror_kernel<<<(c->nc * 32 + 255) / 256, 256, 0, c->stream>>>(c->Scc.p, SA.bsr, c->cols.p, c->nc); LAUNCH_CHECK();
-    c->launches += 2;
+    c->launches += 1;
     finish_cam_kernel<<<(c->nc + 63) / 64, 64, 0, c->stream>>>(c->Scc.p, SA.bsr, c->lmD_cam.p, m.pose_mask, c->nc, c->Minv_c.p, c->fail.p, use_dense ? 0 : 1); LAUNCH_CHECK();
     finish_intr_kernel<<<1, 256, 0, c->stream>>>(c->Sii.p, c->lmD_intr.p, c->intr_mask.p, c->ni8, c->Minv_i.p, c->work_i.p, c->fail.p, (use_pcg3 || use_dense) ? 0 : 1); LAUNCH_CHECK();
     // ---- PCG on S z = rhs

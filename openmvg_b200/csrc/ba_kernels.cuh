@@ -662,8 +662,7 @@ struct SchurArgs {
   const int *obs_pose, *obs_intr, *obs_pt, *pt_start; const unsigned char *pt_single;
   const double *FtF, *FiFi, *g_cam, *g_intr;
   long long n; int n_poses, n_intr, pts_free, kiu;
-  int n_points;     // schur_pair_kernel: landmarks
-  int skip_fast;    // schur_kernel: leave the landmarks the split Schur step handles (pt_single and <= 32 observations) alone
+  int skip_fast;   // schur_kernel: leave the landmarks the split Schur step handles (pt_single and <= 32 observations) alone
   Bsr bsr;
   double *Scc;      // [nnzb][36]
   double *Sci;      // [KI*n_intr][6*n_poses]
@@ -675,18 +674,20 @@ struct SchurArgs {
 
 // Radius-independent part of the reduced system, computed once per Jacobian evaluation without atomics
 // (cam_colsum / intr_colsum): Scc(p,p) = Fc'Fc, Sii(q,q) = Fi'Fi, rhs = [Fc'r ; Fi'r].  S must be zeroed first.
+// With the points eliminated schur_gather_kernel writes all of Scc, Fc'Fc included, and Scc is left alone here.
 __global__ void s_init_kernel(SchurArgs A) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const int nc36 = 36 * A.n_poses, ni64 = 64 * A.n_intr, nred = 6 * A.n_poses + KI * A.n_intr;
-  if (i < nc36) { const int p = i / 36; A.Scc[36 * (size_t)bsr_find(A.bsr, p, p) + i % 36] = A.FtF[i]; }
+  if (i < nc36 && !A.pts_free) { const int p = i / 36; A.Scc[36 * (size_t)bsr_find(A.bsr, p, p) + i % 36] = A.FtF[i]; }
   if (i < ni64) { const int q = i / 64, e = i % 64; A.Sii[(size_t)(KI * q + e / KI) * (KI * A.n_intr) + KI * q + e % KI] = A.FiFi[i]; }
   if (i < nred) A.rhs[i] = i < 6 * A.n_poses ? A.g_cam[i] : A.g_intr[i - 6 * A.n_poses];
 }
 
 // One thread per observation t.  Adds the point-elimination terms  -(E'F)' (E'E + D^2)^-1 (E'F)  and the
-// same-observation border term Fi'Fc.  Camera-pair blocks are accumulated for cam(u) >= cam(t) only
-// (mirror_kernel fills the lower triangle); everything hot (the intrinsics corner, its right-hand side) is
-// reduced per point first so that no address sees more than ~one atomic per point.
+// same-observation border term Fi'Fc.  Camera-pair blocks are visited for cam(u) >= cam(t) and the term goes to both
+// (cam(t), cam(u)) and its transpose: it adds to what schur_gather_kernel wrote, which is both triangles.  Everything
+// hot (the intrinsics corner, its right-hand side) is reduced per point first so that no address sees more than ~one
+// atomic per point.
 constexpr int SCHUR_THREADS = 128;
 __global__ void __launch_bounds__(SCHUR_THREADS) schur_kernel(SchurArgs A) {
   __shared__ double s_ii[KI * KI + KI];
@@ -791,12 +792,17 @@ __global__ void __launch_bounds__(SCHUR_THREADS) schur_kernel(SchurArgs A) {
         for (int a = 0; a < 3; ++a)
           #pragma unroll
           for (int c = 0; c < 6; ++c) efu[a * 6 + c] = up[a] * uc[c] + up[3 + a] * uc[6 + c];
-        if (cu >= ct) {                                        // Scc(ct, cu) -= (Einv E'Fc_t)' E'Fc_u
+        if (cu >= ct) {                                        // Scc(ct, cu) -= (Einv E'Fc_t)' E'Fc_u, and Scc(cu, ct) its transpose
           double *blk = A.Scc + 36 * (size_t)bsr_find(A.bsr, ct, cu);
+          double *blt = cu > ct ? A.Scc + 36 * (size_t)bsr_find(A.bsr, cu, ct) : nullptr;
           #pragma unroll
           for (int a = 0; a < 6; ++a)
             #pragma unroll
-            for (int b = 0; b < 6; ++b) atomicAdd(&blk[a * 6 + b], -(gt_c[a] * efu[b] + gt_c[6 + a] * efu[6 + b] + gt_c[12 + a] * efu[12 + b]));
+            for (int b = 0; b < 6; ++b) {
+              const double v = -(gt_c[a] * efu[b] + gt_c[6 + a] * efu[6 + b] + gt_c[12 + a] * efu[12 + b]);
+              atomicAdd(&blk[a * 6 + b], v);
+              if (blt) atomicAdd(&blt[b * 6 + a], v);
+            }
         }
         if (!single) {
           const int qu = A.obs_intr[u];
@@ -829,14 +835,12 @@ __global__ void __launch_bounds__(SCHUR_THREADS) schur_kernel(SchurArgs A) {
 
 constexpr int CORNER_REPS = 64;
 
-// ---- warp-per-landmark Schur step for the common landmark (all its observations through one intrinsic group, at most
-// 32 of them), in two kernels: the staging half needs ~160 registers, the pair walk ~40; fused into one kernel the walk
-// ran at 12-20 warps per SM and was latency-bound (0.94 ms).
-//   schur_stage_kernel : thread per observation (coalesced component-major loads), per-observation border / rhs
-//                        terms, writes GE[obs] = { Einv E'Fc (18), E'Fc (18) }  (288 B per observation)
-//   schur_pair_kernel  : warp per landmark, lane e adds element e of block (cam_t, cam_u) reading GE through L1: one RED
-//                        instruction touches the 9 sectors of one block instead of 32 sectors of 32 different blocks
-//                        (measured on B200, tools/atomic_bench.cu: 565 vs 222 G FP64 atomics/s)
+// ---- Schur step for the common landmark (all its observations through one intrinsic group, at most 32 of them), in
+// two kernels:
+//   schur_stage_kernel  : thread per observation (coalesced component-major loads), per-observation border / rhs
+//                         terms, writes GE[obs] = { Einv E'Fc (18), E'Fc (18) }  (288 B per observation)
+//   schur_gather_kernel : warp per upper block of Scc, sums the block's terms from GE over the pair lists built at
+//                         create and stores the block and its transpose once (no atomics, fixed order)
 // KIU = intrinsic columns in use (3 pinhole .. 8 Brown): the generic 8-column body kept 16 Jacobian and 24 EtFi values
 // live per thread (162 registers, 3 CTAs per SM, 17 % of the warps active, 5x off its DRAM time).  The 36 doubles of an
 // observation's {E^-1 E'F, E'F} record go through shared memory so that a warp writes its 32 records (9 KB, contiguous)
@@ -937,58 +941,98 @@ __global__ void corner_fold_kernel(const double *__restrict__ corner_rep, const 
   if (e < KI * KI) atomicAdd(&Sii[(size_t)(KI * q0 + e / KI) * ni8 + KI * q0 + e % KI], v);
   else atomicAdd(&rhs[6 * n_poses + KI * q0 + (e - KI * KI)], v);
 }
-__global__ void __launch_bounds__(256) schur_pair_kernel(SchurArgs A, const double *__restrict__ GE) {
-  const int lane = threadIdx.x & 31;
-  const int gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
-  const int ea = lane / 6, eb2 = lane % 6, fa = (32 + lane) / 6, fb = (32 + lane) % 6;
-  // GE (288 MB at 1M observations) comes from DRAM: the lines of a landmark (K x 288 B) are prefetched into L1 one
-  // landmark ahead, otherwise every first touch inside the pair walk is an exposed ~1 us miss
-  int t0n = 0, Kn = 0;
-  if (gwarp < A.n_points) { t0n = A.pt_start[gwarp]; Kn = A.pt_start[gwarp + 1] - t0n; }
-  { const char *pf = reinterpret_cast<const char *>(GE + 36 * (size_t)t0n) + 128 * lane;
-    if (128 * lane < 288 * Kn) asm volatile("prefetch.global.L1 [%0];" :: "l"(pf)); if (128 * (lane + 32) < 288 * Kn) asm volatile("prefetch.global.L1 [%0];" :: "l"(pf + 4096)); }
-  for (int j = gwarp; j < A.n_points; j += nwarps) {
-    const int t0 = t0n, K = Kn;
-    if (j + nwarps < A.n_points) {
-      t0n = A.pt_start[j + nwarps]; Kn = A.pt_start[j + nwarps + 1] - t0n;
-      const char *pf = reinterpret_cast<const char *>(GE + 36 * (size_t)t0n) + 128 * lane;
-      if (128 * lane < 288 * Kn) asm volatile("prefetch.global.L1 [%0];" :: "l"(pf)); if (128 * (lane + 32) < 288 * Kn && Kn <= 32) asm volatile("prefetch.global.L1 [%0];" :: "l"(pf + 4096));
-    }
-    if (K == 0 || K > 32 || !A.pt_single[j]) continue;
-    const int cam_l = lane < K ? A.obs_pose[t0 + lane] : 0;
-    const unsigned lowmask = (1u << (cam_l & 31)) - 1u;
-    int rp = 0, wp = 0; unsigned bm = 0;
-    { const int c0 = __shfl_sync(0xffffffffu, cam_l, 0); const size_t w = (size_t)c0 * A.bsr.words + (cam_l >> 5); rp = A.bsr.rowptr[c0]; wp = A.bsr.wprefix[w]; bm = A.bsr.bitmap[w]; }
-    const double *ge = GE + 36 * (size_t)t0;
-    for (int tt = 0; tt < K; ++tt) {
-      const int ctt = __shfl_sync(0xffffffffu, cam_l, tt);
-      const int cur = (lane < K && cam_l >= ctt) ? rp + wp + __popc(bm & lowmask) : -1;
-      if (tt + 1 < K) { const int cn = __shfl_sync(0xffffffffu, cam_l, tt + 1); const size_t w = (size_t)cn * A.bsr.words + (cam_l >> 5); rp = A.bsr.rowptr[cn]; wp = A.bsr.wprefix[w]; bm = A.bsr.bitmap[w]; }
-      const double *gt = ge + 36 * tt;
-      const double g0 = gt[ea], g1 = gt[6 + ea], g2 = gt[12 + ea];
-      const double h0 = lane < 4 ? gt[fa] : 0.0, h1 = lane < 4 ? gt[6 + fa] : 0.0, h2 = lane < 4 ? gt[12 + fa] : 0.0;
-      unsigned todo = __ballot_sync(0xffffffffu, cur >= 0);
-      while (todo) {
-        const int u = __ffs(todo) - 1; todo &= todo - 1;
-        const int bi = __shfl_sync(0xffffffffu, cur, u);
-        double *blk = A.Scc + 36 * (size_t)bi;
-        const double *ef = ge + 36 * u + 18;
-        atomicAdd(blk + lane, -(g0 * ef[eb2] + g1 * ef[6 + eb2] + g2 * ef[12 + eb2]));
-        if (lane < 4) atomicAdd(blk + 32 + lane, -(h0 * ef[fb] + h1 * ef[6 + fb] + h2 * ef[12 + fb]));
-      }
+// ---- pair lists of schur_gather_kernel, built once per context (omvg_ba_create).  An entry is one term of the
+// split Schur step: a landmark j the warp-per-landmark step takes (pt_single, 1..32 observations) and two of its
+// observations t, u with cam(t) <= cam(u), t = u included.  Entries are grouped by the upper Scc block (cam(t), cam(u)),
+// in the order of the work list (wpos), and kept in landmark order inside a group (stable radix sort).  Observation
+// weights, fixed and removed landmarks do not change the lists: GE carries them.
+__device__ __forceinline__ bool pair_fast(const int *__restrict__ pt_start, const unsigned char *__restrict__ pt_single, int j, int &t0, int &K) {
+  t0 = pt_start[j]; K = pt_start[j + 1] - t0;
+  return pt_single[j] != 0 && K >= 1 && K <= 32;
+}
+__global__ void pair_count_kernel(const int *__restrict__ pt_start, const unsigned char *__restrict__ pt_single, const int *__restrict__ obs_pose,
+                                  int n_points, long long *__restrict__ count) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x; if (j > n_points) return;
+  long long cnt = 0; int t0, K;
+  if (j < n_points && pair_fast(pt_start, pt_single, j, t0, K))
+    for (int t = 0; t < K; ++t) { const int ct = obs_pose[t0 + t]; for (int u = 0; u < K; ++u) cnt += obs_pose[t0 + u] >= ct; }
+  count[j] = cnt;                                    // count[n_points] = 0: the exclusive scan then ends in the total
+}
+__global__ void pair_fill_kernel(const int *__restrict__ pt_start, const unsigned char *__restrict__ pt_single, const int *__restrict__ obs_pose,
+                                 int n_points, const long long *__restrict__ offs, Bsr B, const int *__restrict__ wpos,
+                                 int *__restrict__ key, unsigned long long *__restrict__ pair) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x; if (j >= n_points) return;
+  int t0, K; if (!pair_fast(pt_start, pt_single, j, t0, K)) return;
+  long long o = offs[j];
+  for (int t = 0; t < K; ++t) {
+    const int ct = obs_pose[t0 + t];
+    for (int u = 0; u < K; ++u) {
+      const int cu = obs_pose[t0 + u]; if (cu < ct) continue;
+      key[o] = wpos[bsr_find(B, ct, cu)];
+      pair[o] = ((unsigned long long)(unsigned)(t0 + u) << 32) | (unsigned)(t0 + t);   // int2 {t, u}
+      ++o;
     }
   }
 }
 
-// lower triangle of Scc from the upper one: block (a,b), a > b, = block (b,a)'
-__global__ void mirror_kernel(double *__restrict__ Scc, Bsr B, const int *__restrict__ cols, int n_poses) {
-  const int a = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-  if (a >= n_poses) return;
-  for (int e = B.rowptr[a]; e < B.rowptr[a + 1]; ++e) {
-    const int b = cols[e]; if (b >= a) break;
-    const double *src = Scc + 36 * (size_t)bsr_find(B, b, a); double *dst = Scc + 36 * (size_t)e;
-    for (int k = lane; k < 36; k += 32) dst[k] = src[(k % 6) * 6 + k / 6];
+// Scc(a, b) for every upper block (a <= b) of the work list and its transpose:  Fc'Fc (a = b)  -  sum over the block's
+// entries of (Einv E'Fc_t)' E'Fc_u, each entry read from the GE records of schur_stage_kernel.  One warp per block; lane l
+// takes entries l, l + 32, ... and accumulates all 36 elements in registers (18 16-byte loads per entry per lane, against
+// 12 8-byte loads per entry per WARP lane if lanes split the block's elements), then the 32 partial blocks are reduced by
+// a fixed shuffle tree.  Every block is written, empty ones included, so Scc needs no zeroing; with no landmark on the
+// per-observation path the result does not depend on scheduling.
+constexpr int GATHER_THREADS = 128;
+__global__ void __launch_bounds__(GATHER_THREADS) schur_gather_kernel(const double *__restrict__ GE, const int *__restrict__ gstart, const int2 *__restrict__ pairs,
+                                                                      const int *__restrict__ gblk, const int *__restrict__ gblkT, int nwork,
+                                                                      const int *__restrict__ brow, const double *__restrict__ FtF, double *__restrict__ Scc) {
+  const int w = (int)(((long long)blockIdx.x * GATHER_THREADS + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (w >= nwork) return;                           // (whole warps: nwork is a warp count)
+  double acc[36];
+  #pragma unroll
+  for (int i = 0; i < 36; ++i) acc[i] = 0.0;
+  const int e1 = gstart[w + 1];
+  for (int e = gstart[w] + lane; e < e1; e += 32) {
+    const int2 pr = pairs[e];
+    const double2 *g2 = reinterpret_cast<const double2 *>(GE + 36 * (size_t)pr.x);        // Einv E'Fc_t (3 x 6)
+    const double2 *f2 = reinterpret_cast<const double2 *>(GE + 36 * (size_t)pr.y + 18);   // E'Fc_u (3 x 6)
+    double g[18], f[18];
+    #pragma unroll
+    for (int k = 0; k < 9; ++k) { const double2 v = g2[k]; g[2 * k] = v.x; g[2 * k + 1] = v.y; }
+    #pragma unroll
+    for (int k = 0; k < 9; ++k) { const double2 v = f2[k]; f[2 * k] = v.x; f[2 * k + 1] = v.y; }
+    #pragma unroll
+    for (int a = 0; a < 3; ++a)
+      #pragma unroll
+      for (int r = 0; r < 6; ++r)
+        #pragma unroll
+        for (int c = 0; c < 6; ++c) acc[r * 6 + c] = fma(g[a * 6 + r], f[a * 6 + c], acc[r * 6 + c]);
   }
+  // reduce-scatter over lane bits 4 and 3 (36 -> 18 -> 9 elements per lane), then a butterfly over bits 2..0: the 8
+  // lanes of group q = lane >> 3 hold the block's elements 9q .. 9q + 8, summed over all 32 lanes
+  double h[18], v[9];
+  { const bool up = lane & 16;
+    #pragma unroll
+    for (int i = 0; i < 18; ++i) { const double keep = up ? acc[18 + i] : acc[i], send = up ? acc[i] : acc[18 + i]; h[i] = keep + __shfl_xor_sync(0xffffffffu, send, 16); } }
+  { const bool up = lane & 8;
+    #pragma unroll
+    for (int i = 0; i < 9; ++i) { const double keep = up ? h[9 + i] : h[i], send = up ? h[i] : h[9 + i]; v[i] = keep + __shfl_xor_sync(0xffffffffu, send, 8); } }
+  #pragma unroll
+  for (int m = 4; m >= 1; m >>= 1)
+    #pragma unroll
+    for (int i = 0; i < 9; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], m);
+  const int s = lane & 7, q = lane >> 3;
+  double x = v[0];
+  #pragma unroll
+  for (int i = 1; i < 8; ++i) if (s == i) x = v[i];
+  const int eu = gblk[w], el = gblkT[w];
+  const double *ftf = FtF + 36 * (size_t)brow[eu];
+  auto put = [&](int idx, double sum) {
+    if (eu == el) { Scc[36 * (size_t)eu + idx] = ftf[idx] - sum; return; }
+    Scc[36 * (size_t)eu + idx] = -sum;
+    Scc[36 * (size_t)el + (idx % 6) * 6 + idx / 6] = -sum;
+  };
+  put(9 * q + s, x);
+  if (s == 0) put(9 * q + 8, v[8]);
 }
 
 // S diag += D^2 (free columns) / = 1 (masked columns); block-Jacobi preconditioner Minv_c = inv(diag block)
